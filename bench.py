@@ -3,6 +3,7 @@
 exploration sets) on N GPUs of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--sets-per-gpu S] [--strong [--sets T]]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -53,7 +54,14 @@ def parse():
     ap.add_argument("--direct-candidates", type=int, default=None,
                     help="candidates timed in the reference-faithful one-at-a-time form (default: 16 in the reference arm, 2 in cpu_baseline)")
     ap.add_argument("--strict-selection", action="store_true", help="exit non-zero when the selected intervention differs from profiles/expected_selection.json")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float64; see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 ARGS = parse()
@@ -223,6 +231,7 @@ class ClockSampler(threading.Thread):
     def stop(self):
         if self.proc is not None:
             self.proc.terminate()
+            self.proc.wait()
         sm = [float(r[1]) for r in self.rows if len(r) >= 9 and r[1].replace(".", "").isdigit()]
         mx = [float(r[2]) for r in self.rows if len(r) >= 9 and r[2].replace(".", "").isdigit()]
         reasons = set()
@@ -249,11 +258,17 @@ def emit(line):
 
 def measure_fp64_peak(gpu_index):
     """FP64 DMMA issue rate of THIS box, measured before the timed region with the micro-benchmark of tools/fp64_peak.cu
-    (built by __graft_entry__.build(); compiled here if the binary did not travel).  Falls back to the round-1 measurement."""
+    (built by __graft_entry__.build(); otherwise compiled into a temporary directory: the tree may be read-only).  Falls back to
+    the round-1 measurement."""
+    import tempfile
+    from cbo_with_oop_b200.build import _nvcc
     exe = os.path.join(ROOT, "tools", "fp64_peak")
+    tmp = None
     try:
         if not os.path.exists(exe):
-            subprocess.check_call(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-o", exe,
+            tmp = tempfile.TemporaryDirectory(prefix="cbo_fp64_peak_")
+            exe = os.path.join(tmp.name, "fp64_peak")
+            subprocess.check_call([_nvcc(), "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-o", exe,
                                    os.path.join(ROOT, "tools", "fp64_peak.cu")], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         env = dict(os.environ, CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", "").split(",")[gpu_index]
                    if os.environ.get("CUDA_VISIBLE_DEVICES") else str(gpu_index))
@@ -268,6 +283,41 @@ def measure_fp64_peak(gpu_index):
                 "round-1 measurement on this pool's B200 (profiles/fp64_peak_r01.json); the in-run probe failed: %s" % type(e).__name__
         except Exception:  # noqa: BLE001
             return 36.97, "fallback constant (round-1 measurement)"
+    finally:
+        if tmp is not None:
+            tmp.cleanup()
+
+
+DUMP_SAMPLE = 1 << 20      # candidates whose posterior is written, over all sets: 4 arrays x 8 B x 2^20 = 32 MB
+
+
+def dump_outputs(path, eng, out):
+    """Write what one SweepEngine.sweep computed as float64 .npy files under `path` (about 32 MB at most), so that two
+    builds can be compared output for output on the same seeded inputs:
+      selected.npy                         [set, flat index, acquisition value, NaN count] of the next intervention
+      selected_x.npy                       its coordinates
+      set_values.npy, set_indices.npy      every exploration set's best acquisition value and its flat index
+      sample_set.npy, sample_index.npy,    posterior mean and variance (the device arrays the sweep leaves behind) at a
+      mu.npy, var.npy                      fixed seeded sample of each set's candidates, or at all of them when they fit
+    Only candidates this rank holds are written; which ones are sampled does not depend on the partition."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"selected": [out.set, out.index, out.value, out.n_nan],
+              "selected_x": out.x if out.x is not None else np.zeros(0),
+              "set_values": out.set_values, "set_indices": out.set_indices}
+    per_set = DUMP_SAMPLE // len(eng.problems)
+    cols = {"sample_set": [], "sample_index": [], "mu": [], "var": []}
+    for g in eng.active:
+        G = eng.problems[g].g_total
+        idx = np.arange(G) if G <= per_set else np.sort(np.random.default_rng([0, g]).choice(G, per_set, replace=False))
+        gb, gc = eng.slices[g]
+        idx = idx[(idx >= gb) & (idx < gb + gc)]
+        cols["sample_set"].append(np.full(len(idx), g))
+        cols["sample_index"].append(idx)
+        for k in ("mu", "var"):
+            cols[k].append(eng.fetch(k, g)[idx - gb])
+    arrays.update({k: np.concatenate(v) if v else np.zeros(0) for k, v in cols.items()})
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def timed_trials(eng, best, dev, n, warm):
@@ -396,8 +446,12 @@ def run_ours(args, world, rank, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms, out, stage_ms, launches, _ = timed(eng, best, args.steps, False)
-    clocks = sampler.stop() if rank == 0 else None
+    try:
+        ms, out, stage_ms, launches, _ = timed(eng, best, args.steps, False)
+    finally:
+        clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:     # before the post-intervention trials below overwrite mu / var
+        dump_outputs(args.dump_outputs, eng, out)
     total_pts = S * G_set
     value = total_pts / (ms / args.steps * 1e-3)
 

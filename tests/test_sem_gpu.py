@@ -51,14 +51,12 @@ def test_device_sem_matches_shipped_true_effects(cuda_engine_ready):
     assert np.abs(got - np.asarray(row[4], np.float64).reshape(-1)).max() < 0.05
 
 
-def test_monitor_uses_the_device_simulator(cuda_engine_ready):
-    import os
+def test_monitor_uses_the_device_simulator(cuda_engine_ready, tmp_path, monkeypatch):
     import types
     from src.CBO import CBO
     from src.DataLoader import DataLoader
     from src.utils_functions.graph_functions import compute_interventions
-    os.makedirs("/tmp/cbo_test_out", exist_ok=True)
-    os.chdir("/tmp/cbo_test_out")
+    monkeypatch.chdir(tmp_path)          # the agent creates ./data/<experiment>/... for its results
     args = types.SimpleNamespace(exploration_set="MIS", initial_num_obs_samples=60, num_interventions=10, type_cost=1,
                                  num_additional_observations=20, num_trials=3, name_index=0, seed=9, causal_prior=True,
                                  experiment="complete_graph", task="min", grid_points=20, device="cuda:0", num_sem_samples=5000)

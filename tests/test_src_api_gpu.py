@@ -13,11 +13,15 @@ from oracle import cbo_oracle as O
 pytestmark = pytest.mark.gpu
 
 
-def make_agent(experiment="toy_graph", n_obs=60, trials=4, causal=True, p=40, tmp="/tmp/cbo_test_out"):
+@pytest.fixture(autouse=True)
+def in_tmp(tmp_path, monkeypatch):
+    """The agent saves its results under ./data/: keep them in a per-test directory."""
+    monkeypatch.chdir(tmp_path)
+
+
+def make_agent(experiment="toy_graph", n_obs=60, trials=4, causal=True, p=40):
     from src.CBO import CBO
     from src.DataLoader import DataLoader
-    os.makedirs(tmp, exist_ok=True)
-    os.chdir(tmp)
     args = types.SimpleNamespace(exploration_set="MIS", initial_num_obs_samples=n_obs, num_interventions=10, type_cost=1,
                                  num_additional_observations=20, num_trials=trials, name_index=0, seed=9, causal_prior=causal,
                                  experiment=experiment, task="min", grid_points=p, device="cuda:0", num_sem_samples=2000)
