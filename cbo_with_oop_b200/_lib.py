@@ -8,7 +8,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CBO_B200_LIB") or os.path.join(HERE, "libcbo_b200.so")   # (the override is for kernel experiments)
 
-CBO_ABI_VERSION = 6
+CBO_ABI_VERSION = 7
 CBO_MAX_D = 4
 CBO_MAX_C = 8
 CBO_MAX_NINT = 128
@@ -49,13 +49,29 @@ class SweepResult(C.Structure):
     _fields_ = [("value", C.c_double), ("index", C.c_int64), ("set", C.c_int32), ("n_nan", C.c_int32)]
 
 
+class AcqGradOut(C.Structure):
+    """Mirror of cbo_acq_grad_out (value and gradient of the acquisition at one point)."""
+    _fields_ = [(n, C.c_double) for n in ("m", "v", "mu", "var", "ei", "acq")] + \
+               [(n, C.c_double * CBO_MAX_D) for n in ("dm", "dv", "dmu", "dvar", "dei", "dacq")]
+
+
+class RefineResult(C.Structure):
+    """Mirror of cbo_refine_result (one exploration set's refined maximum)."""
+    _fields_ = [("x", C.c_double * CBO_MAX_D), ("value", C.c_double), ("start_value", C.c_double),
+                ("iterations", C.c_int32), ("status", C.c_int32)]
+
+
+REFINE_STATUS = {0: "converged", 1: "max_iter", 2: "line_search_failed", 3: "skipped_external_prior",
+                 4: "skipped_explicit_points", 5: "skipped_nonfinite"}
+
 EXPORTS = [
     "cbo_abi_version", "cbo_sizeof_set_desc", "cbo_offsetof_set_desc", "cbo_last_error", "cbo_sweep_num_items",
     "cbo_prior_workspace_bytes", "cbo_launch_count", "cbo_obs_gp_workspace_bytes", "cbo_prior_pair_items",
     "cbo_prior_eval_flops",
     "cbo_obs_gp_fit", "cbo_obs_gp_nll",
     "cbo_build_tables", "cbo_prior_precompute", "cbo_prior_eval", "cbo_posterior_fit", "cbo_sweep",
-    "cbo_argmax_combine", "cbo_sem_eval", "cbo_refresh_trial",
+    "cbo_argmax_combine", "cbo_sem_eval", "cbo_refresh_trial", "cbo_acq_grad", "cbo_refine",
+    "cbo_refine_workspace_bytes",
 ]
 CBO_SEM_MAX_NODES, CBO_SEM_MAX_TERMS, CBO_SEM_BLOCKS = 16, 96, 64
 SEM_FUNCS = {"id": 0, "exp": 1, "cos": 2, "sin": 3, "square": 4}
@@ -118,8 +134,14 @@ def load() -> C.CDLL:
                                       C.c_void_p, C.c_void_p, C.c_void_p]
     lib.cbo_sem_eval.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_longlong, C.c_void_p, C.c_void_p,
                                  C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.cbo_acq_grad.argtypes = [P, C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p,
+                                 C.c_void_p]
+    lib.cbo_refine.argtypes = [P, C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_int, C.c_double, C.c_void_p,
+                               C.c_size_t, C.c_void_p, C.c_void_p]
     for name in EXPORTS[10:]:
         getattr(lib, name).restype = C.c_int
+    lib.cbo_refine_workspace_bytes.restype = C.c_size_t
+    lib.cbo_refine_workspace_bytes.argtypes = [P, C.c_int]
     if lib.cbo_abi_version() != CBO_ABI_VERSION:
         raise ImportError(f"ABI version mismatch: library {lib.cbo_abi_version()} != binding {CBO_ABI_VERSION}")
     if lib.cbo_sizeof_set_desc() != C.sizeof(SetDesc):

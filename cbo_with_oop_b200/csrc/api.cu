@@ -71,6 +71,10 @@ size_t obs_gp_workspace_bytes_impl(const cbo_set_desc*, int);
 int obs_gp_fit_impl(const cbo_set_desc*, int, double, void*, size_t, int32_t*, cudaStream_t);
 int obs_gp_nll_impl(const cbo_set_desc*, void*, size_t, double*, cudaStream_t);
 int int_rows_table_impl(const cbo_set_desc&, cudaStream_t);
+size_t refine_workspace_bytes_impl(const cbo_set_desc*, int);
+int acq_grad_impl(const cbo_set_desc*, const cbo_set_desc*, const double*, int, double, int, void*, size_t, cbo_acq_grad_out*, cudaStream_t);
+int refine_impl(const cbo_set_desc*, const cbo_set_desc*, int, double, int, const double*, int, double, void*, size_t, cbo_refine_result*,
+                cudaStream_t);
 int sem_eval_impl(const cbo_sem_node*, int, const cbo_sem_term*, int, const double*, int, long long, const int32_t*, const double*, int,
                   int, double*, double*, cudaStream_t);
 
@@ -204,6 +208,24 @@ int cbo_argmax_combine(const cbo_set_best* d_gathered, int num_ranks, int num_se
                        cbo_sweep_result* d_result, void* stream) {
     CBO_REQUIRE(d_set_best && d_result, "cbo_argmax_combine: NULL output pointer");
     return argmax_combine_impl(d_gathered, num_ranks, num_sets, d_set_best, d_result, (cudaStream_t)stream);
+}
+
+size_t cbo_refine_workspace_bytes(const cbo_set_desc* h_sets, int num_sets) {
+    if (!h_sets || num_sets < 1) return 0;
+    return refine_workspace_bytes_impl(h_sets, num_sets);
+}
+
+int cbo_acq_grad(const cbo_set_desc* h_set, const cbo_set_desc* d_set, const double* d_points, int num_points, double best, int task_sign,
+                 void* d_workspace, size_t workspace_bytes, cbo_acq_grad_out* d_out, void* stream) {
+    if (int rc = validate_sets(h_set, 1)) return rc;
+    return acq_grad_impl(h_set, d_set, d_points, num_points, best, task_sign, d_workspace, workspace_bytes, d_out, (cudaStream_t)stream);
+}
+
+int cbo_refine(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, double best, int task_sign, const double* d_x0,
+               int max_iter, double gtol, void* d_workspace, size_t workspace_bytes, cbo_refine_result* d_out, void* stream) {
+    if (int rc = validate_sets(h_sets, num_sets)) return rc;
+    return refine_impl(h_sets, d_sets, num_sets, best, task_sign, d_x0, max_iter, gtol, d_workspace, workspace_bytes, d_out,
+                       (cudaStream_t)stream);
 }
 
 int cbo_sem_eval(const cbo_sem_node* d_nodes, int num_nodes, const cbo_sem_term* d_terms, int num_terms, const double* d_noise,

@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import SetBest, SetDesc, SweepResult
+from ._lib import AcqGradOut, RefineResult, SetBest, SetDesc, SweepResult
 from .partition import SetSize, partition
 
 
@@ -97,6 +97,10 @@ class SweepOutput:
     set_indices: np.ndarray  # (S,) flat index of each set's best candidate
     n_nan: int
     stage_ms: Dict[str, float] = field(default_factory=dict)
+    # filled by SweepEngine.refine: per-set coordinates of set_values ((d_s,) each; None for a set without a maximum) and
+    # the per-set outcome of the refinement (_lib.REFINE_STATUS names)
+    set_x: Optional[List[Optional[np.ndarray]]] = None
+    refine_status: Optional[List[str]] = None
 
 
 def _round_up(x: int, m: int) -> int:
@@ -638,6 +642,104 @@ class SweepEngine:
             for k in names:
                 out[k][a:a + mc] = bufs[k].cpu().numpy()
         return out
+
+    # ------------------------------------------------------------------------------------------------
+    _GRAD_DTYPE = np.dtype([(n, "f8") for n in ("m", "v", "mu", "var", "ei", "acq")] +
+                           [(n, "f8", (_lib.CBO_MAX_D,)) for n in ("dm", "dv", "dmu", "dvar", "dei", "dacq")])
+
+    def _local_desc(self, li: int):
+        self._push_descs()
+        h = C.cast(C.byref(self.h_sets, li * C.sizeof(SetDesc)), C.POINTER(SetDesc))
+        return h, C.c_void_p(self.d_sets.data_ptr() + li * C.sizeof(SetDesc))
+
+    def _refine_workspace(self, nbytes: int) -> torch.Tensor:
+        """K7's workspace, grown on demand and kept (stream-ordered reuse)."""
+        ws = getattr(self, "_refine_ws", None)
+        if ws is None or ws.numel() < nbytes:
+            ws = torch.empty((max(nbytes, 256),), dtype=torch.uint8, device=self.device)
+            self._refine_ws = ws
+        return ws
+
+    def acquisition_gradients(self, g: int, X: np.ndarray, best: float = 0.0, task: str = "min") -> Dict[str, np.ndarray]:
+        """Value and gradient with respect to x of the prior, posterior, EI and EI / cost of global set g at the rows of X
+        (m, d), with the set's CURRENT device state (cbo_acq_grad, K7): the gradient behind
+        CausalExpectedImprovement.evaluate_with_gradients (causal_acquisition_functions.py:45-67).  Scalars come back with
+        shape (m,), gradients (dm, dv, dmu, dvar, dei, dacq) with shape (m, d)."""
+        if task not in ("min", "max"):
+            raise ValueError("task must be 'min' or 'max'")
+        li = self.local_of[g]
+        pr = self.problems[g]
+        X = np.ascontiguousarray(np.asarray(X, np.float64).reshape(-1, pr.d))
+        m = X.shape[0]
+        if m == 0:
+            return {n: np.empty((0,) + ((pr.d,) if n.startswith("d") else ())) for n in self._GRAD_DTYPE.names}
+        h, dptr = self._local_desc(li)
+        one = self.lib.cbo_refine_workspace_bytes(h, 1)
+        ws = self._refine_workspace(one * min(16, (m + 7) // 8))
+        pts = torch.from_numpy(X.reshape(-1)).to(self.device)
+        out = torch.empty((m * C.sizeof(AcqGradOut),), dtype=torch.uint8, device=self.device)
+        _lib.check(self.lib.cbo_acq_grad(h, dptr, C.c_void_p(pts.data_ptr()), m, float(best), 1 if task == "min" else -1,
+                                         C.c_void_p(ws.data_ptr()), ws.numel(), C.c_void_p(out.data_ptr()), self._stream()),
+                   "cbo_acq_grad")
+        rec = np.frombuffer(out.cpu().numpy().tobytes(), dtype=self._GRAD_DTYPE)
+        return {n: (rec[n][:, :pr.d].copy() if n.startswith("d") else rec[n].copy()) for n in self._GRAD_DTYPE.names}
+
+    def refine(self, out: SweepOutput, best: float, task: str = "min", max_iter: int = 30, gtol: float = 1e-7) -> SweepOutput:
+        """Refine every set's acquisition maximum off the grid (cbo_refine, K7): a projected quasi-Newton ascent of EI / cost
+        inside the set's box [min grid[k], max grid[k]], started at the set's grid argmax in `out` (the output of the sweep
+        that left the current device state).  Replaces the L-BFGS polish of the reference's anchor search
+        (causal_optimizer.py:52-62).  Returns a copy of `out` whose set_values, set_x and refine_status are per set and whose
+        set / value / x are chosen by the sweep's rule (first maximum, NaN = -inf); `index` stays the grid index the chosen
+        set started from.  A set that is skipped (external prior, explicit points, no finite grid maximum) or that no step
+        improved keeps its grid index, value and coordinates bit for bit."""
+        if self.world > 1:
+            raise ValueError("refine runs on one GPU: a multi-GPU engine would need the refined per-set results all-gathered")
+        if task not in ("min", "max"):
+            raise ValueError("task must be 'min' or 'max'")
+        S, A = len(self.problems), len(self.active)
+        grid_x = [None] * S
+        for g in range(S):
+            if out.set_indices[g] >= 0:
+                pr = self.problems[g]
+                ii = np.unravel_index(int(out.set_indices[g]), [len(t) for t in pr.grid])
+                grid_x[g] = np.array([pr.grid[k][ii[k]] for k in range(pr.d)])
+        x0 = np.full((max(A, 1), _lib.CBO_MAX_D), np.nan)
+        for li, g in enumerate(self.active):
+            if grid_x[g] is not None and np.isfinite(out.set_values[g]):
+                x0[li, :self.problems[g].d] = grid_x[g]
+        ev: list = []
+        res = None
+        if A:
+            self._push_descs()
+            ws = self._refine_workspace(self.lib.cbo_refine_workspace_bytes(self.h_sets, A))
+            d_x0 = torch.from_numpy(x0.reshape(-1)).to(self.device)
+            d_res = torch.empty((A * C.sizeof(RefineResult),), dtype=torch.uint8, device=self.device)
+            self._timed("refine", lambda: _lib.check(self.lib.cbo_refine(
+                self.h_sets, C.c_void_p(self.d_sets.data_ptr()), A, float(best), 1 if task == "min" else -1,
+                C.c_void_p(d_x0.data_ptr()), int(max_iter), float(gtol), C.c_void_p(ws.data_ptr()), ws.numel(),
+                C.c_void_p(d_res.data_ptr()), self._stream()), "cbo_refine"), ev)
+            res = (RefineResult * A).from_buffer_copy(d_res.cpu().numpy().tobytes())
+        values = np.array(out.set_values, np.float64, copy=True)
+        set_x = list(grid_x)
+        status = ["skipped_nonfinite"] * S
+        for li, g in enumerate(self.active):
+            r = res[li]
+            status[g] = _lib.REFINE_STATUS.get(r.status, str(r.status))
+            if r.value > r.start_value:          # strictly improved (both finite)
+                values[g] = r.value
+                set_x[g] = np.array(r.x[:self.problems[g].d])
+        valid = np.flatnonzero(np.asarray(out.set_indices) >= 0)
+        s, value, x = -1, out.value, None
+        if valid.size:
+            v = np.where(np.isnan(values[valid]), -np.inf, values[valid])
+            s = int(valid[int(np.argmax(v))])
+            value, x = float(values[s]), set_x[s]
+        ms = dict(out.stage_ms)
+        for name, e0, e1 in ev:
+            e1.synchronize()
+            ms[name] = ms.get(name, 0.0) + e0.elapsed_time(e1)
+        return SweepOutput(s, int(out.set_indices[s]) if s >= 0 else out.index, value, x, values,
+                           np.array(out.set_indices, copy=True), out.n_nan, ms, set_x=set_x, refine_status=status)
 
     def fetch(self, name: str, g: int) -> np.ndarray:
         """Device array of global set g as NumPy (parity tests / debugging)."""

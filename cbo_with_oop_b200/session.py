@@ -71,11 +71,21 @@ class AcquisitionSession:
         self._ensure_fit(g)
         return self.engine.evaluate_points(g, X, best=best, task=task, stages="all", m_pts=m_pts, v_pts=v_pts)
 
-    def best_per_set(self, best: float, task: str = "min") -> SweepOutput:
-        """The batched form of CBO.compute_best_acquisition_values (CBO.py:237-260): every set's acquisition maximum."""
-        key = (float(best), task)
+    def gradient_points(self, g: int, X: np.ndarray, best: float = 0.0, task: str = "min") -> Dict[str, np.ndarray]:
+        """Values and x-gradients of the prior, posterior, EI and EI / cost of global set g at the rows of X (cbo_acq_grad)."""
+        self._ensure_fit(g)
+        return self.engine.acquisition_gradients(g, X, best=best, task=task)
+
+    def best_per_set(self, best: float, task: str = "min", refine: bool = False) -> SweepOutput:
+        """The batched form of CBO.compute_best_acquisition_values (CBO.py:237-260): every set's acquisition maximum --
+        on the grid, or with refine=True refined off the grid from the grid maximum (SweepEngine.refine)."""
+        key = (float(best), task, bool(refine))
         if self.grid_ready and not self.stale_fit and self.last_output is not None and self._last_key == key:
             return self.last_output      # nothing changed since the last sweep (per-set callers share one device pass)
+        if refine:
+            out = self.engine.refine(self.best_per_set(best, task), best, task)
+            self._last_key, self.last_output = key, out
+            return out
         self._last_key = key
         if not self.grid_ready:
             out = self.engine.sweep(best, task)

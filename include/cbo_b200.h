@@ -30,7 +30,7 @@ extern "C" {
 #define CBO_API
 #endif
 
-#define CBO_ABI_VERSION 6
+#define CBO_ABI_VERSION 7
 #define CBO_MAX_D 4          /* intervened dimensions per exploration set (reference uses 1..3) */
 #define CBO_MAX_C 8          /* conditioning dimensions of an observational GP */
 #define CBO_MAX_NINT 128     /* interventional rows per set (reference: 10 .. ~50) */
@@ -229,6 +229,50 @@ CBO_API int cbo_refresh_trial(const cbo_set_desc* h_sets, cbo_set_desc* d_sets, 
  * all-gathered buffer never leaves it. */
 CBO_API int cbo_argmax_combine(const cbo_set_best* d_gathered, int num_ranks, int num_sets,
                        cbo_set_best* d_set_best, cbo_sweep_result* d_result, void* stream);
+
+/* K7. Continuous refinement of each exploration set's acquisition maximum (opt-in).
+ * Replaces the reference's L-BFGS polish of the best anchor, causal_optimizer.py:52-62, and the gradient it consumes,
+ * CausalExpectedImprovement.evaluate_with_gradients / Cost (causal_acquisition_functions.py:45-67): the value and gradient
+ * of acq(x) = EI(x) / cost(x) for one set at arbitrary points, and a projected quasi-Newton ascent of acq inside the box
+ * [min grid[k], max grid[k]] that starts at a caller-given point (the grid argmax of a preceding cbo_sweep).
+ * Every iteration is one pass over M's lower block triangle for the set's 8 trial points (value and gradient of the
+ * causal prior, csrc/refine.cu) and one step kernel per set; no host synchronisation except a 4-byte poll of the sets
+ * still running every few iterations.  Results are bit-identical across runs and do not depend on which other sets share
+ * the call.  The device state the sweep left behind is read, never written: M, w, x_obs_int, L, alpha, sqrt_v_int, x_int,
+ * grid. */
+enum {
+    CBO_REFINE_CONVERGED = 0,         /* small projected gradient or a negligible step */
+    CBO_REFINE_MAX_ITER = 1,          /* max_iter iterations done */
+    CBO_REFINE_LINE_SEARCH_FAILED = 2, /* none of the 8 trial steps along the gradient direction raised acq (Armijo) */
+    CBO_REFINE_SKIPPED_EXTERNAL = 3,  /* prior_external: no device prior to differentiate */
+    CBO_REFINE_SKIPPED_POINTS = 4,    /* explicit candidate points (points != NULL): no box */
+    CBO_REFINE_SKIPPED_NONFINITE = 5  /* the start point has a NaN coordinate, or acq there is NaN / +-inf */
+};
+typedef struct cbo_acq_grad_out {      /* one explicit point; d* = gradient with respect to x (entries >= d are 0) */
+    double m, v, mu, var, ei, acq;     /* prior mean / variance, posterior mean / variance (incl. 1e-10), EI, EI / cost */
+    double dm[CBO_MAX_D], dv[CBO_MAX_D], dmu[CBO_MAX_D], dvar[CBO_MAX_D], dei[CBO_MAX_D], dacq[CBO_MAX_D];
+} cbo_acq_grad_out;
+typedef struct cbo_refine_result {     /* one set */
+    double x[CBO_MAX_D];  /* refined point; the start point itself when value <= start_value or the set was skipped */
+    double value;         /* acq(x) (refinement arithmetic); equals start_value when no step improved it */
+    double start_value;   /* acq at the start point in the same arithmetic (NaN when skipped) */
+    int32_t iterations;   /* line searches performed */
+    int32_t status;       /* CBO_REFINE_* */
+} cbo_refine_result;
+/* Workspace of cbo_refine for this descriptor list, and of cbo_acq_grad for one set (which then evaluates its points 8 at
+ * a time, more per launch when the workspace is larger). */
+CBO_API size_t cbo_refine_workspace_bytes(const cbo_set_desc* h_sets, int num_sets);
+/* Value and gradient of the prior, posterior, EI and acq of ONE set at d_points (num_points, d) row-major, with the set's
+ * current device state (causal sets need the prior precompute, every set the posterior fit).  d_out: num_points entries. */
+CBO_API int cbo_acq_grad(const cbo_set_desc* h_set, const cbo_set_desc* d_set, const double* d_points, int num_points,
+                         double best, int task_sign, void* d_workspace, size_t workspace_bytes,
+                         cbo_acq_grad_out* d_out, void* stream);
+/* Refine every set from d_x0 (num_sets, CBO_MAX_D) device doubles; a row holding a NaN skips its set.  max_iter line
+ * searches at most; gtol: stop when max_k |projected d acq / dx_k| (max grid[k] - min grid[k]) <= gtol |acq|.
+ * d_out: num_sets entries.  Sets with prior_external or explicit points are skipped (status says why). */
+CBO_API int cbo_refine(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, double best, int task_sign,
+                       const double* d_x0, int max_iter, double gtol,
+                       void* d_workspace, size_t workspace_bytes, cbo_refine_result* d_out, void* stream);
 
 /* K6. Ground truth of an intervention: E[target | do(...)] of a structural equation model by Monte Carlo.
  * Replaces compute_interventions / sample_from_model / intervene_dict (graph_functions.py:8-77: 100 000 samples in a Python

@@ -26,6 +26,9 @@ class ArgumentParser:
         # build-specific, optional
         self.parser.add_argument("--grid_points", default=100, type=int, help="candidate grid points per dimension")
         self.parser.add_argument("--device", default="cuda:0", type=str, help="CUDA device of the sweep")
+        self.parser.add_argument("--refine_acquisition", action="store_true",
+                                 help="refine each exploration set's grid maximum off the grid with on-device gradients "
+                                      "(the reference's L-BFGS polish); off: the grid argmax")
 
     def parse(self, verbose=False, argv=None):
         args = self.parser.parse_args(argv)

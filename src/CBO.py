@@ -44,6 +44,8 @@ class CBO:
         # where observe() fits the observational GPs: "device" (cbo_obs_gp_fit / cbo_obs_gp_nll, the default) or, on explicit
         # request only, "host" (SciPy; input preparation for machines without a GPU -- the sweep itself has no CPU path)
         self.observational_fit = getattr(args, "observational_fit", "device")
+        # refine each set's grid maximum off the grid (SweepEngine.refine): the reference's continuous L-BFGS polish
+        self.refine_acquisition = bool(getattr(args, "refine_acquisition", False))
 
         self.mean_functions, self.var_functions, self.models = [], [], []
         self.costs = self.graph.get_cost_structure(type_cost=self.type_cost)
@@ -164,8 +166,11 @@ class CBO:
         session = self.get_session()
         for s, model in enumerate(self.models):
             session.mark_interventional(s, model.X, model.Y)
-        out = session.best_per_set(float(current_best), self.task)
-        xs = [session.grid_point(s, out.set_indices[s]).reshape(1, -1) for s in range(self.es_size)]
+        out = session.best_per_set(float(current_best), self.task, refine=self.refine_acquisition)
+        if self.refine_acquisition:
+            xs = [np.asarray(out.set_x[s], np.float64).reshape(1, -1) for s in range(self.es_size)]
+        else:
+            xs = [session.grid_point(s, out.set_indices[s]).reshape(1, -1) for s in range(self.es_size)]
         ys = [np.array([[out.set_values[s]]]) for s in range(self.es_size)]
         self.last_sweep = out
         return xs, ys

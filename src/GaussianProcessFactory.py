@@ -86,8 +86,36 @@ class SurrogateModel:
             v_pts = np.asarray(self.var_function(X), np.float64).reshape(-1)
         return session.predict_points(0, X, best, task, m_pts=m_pts, v_pts=v_pts)
 
-    def grid_argmax(self, tables, best, task, cost_fix=1.0, cost_variable=False):
-        """(max of EI / cost over the tensor grid, its coordinates (d,)): the per-set form of the batched sweep."""
+    @property
+    def has_gradients(self):
+        """x-gradients come from the device prior (DoCalculus closures) or need no prior (non-causal); arbitrary Python
+        mean / variance callables have no gradient."""
+        return not self.causal or self._shared() is not None
+
+    def acquisition_gradients(self, X, best, task):
+        """Values and x-gradients of m, v, mu, var, EI and EI / cost at the rows of X (cbo_acq_grad); gradients (m, d)."""
+        X = np.atleast_2d(np.asarray(X, np.float64))
+        shared = self._shared()
+        if shared is not None:
+            session, g = shared
+            session.mark_interventional(g, self.X, self.Y)
+            return session.gradient_points(g, X, best, task)
+        if self.causal:
+            raise ValueError("gradients need the device prior: this model's mean / variance are arbitrary callables")
+        session = self._private_session([np.zeros(1)] * self.X.shape[1])
+        return session.gradient_points(0, X, best, task)
+
+    def get_prediction_gradients(self, X):
+        """(d mean / dx (m, d), d variance / dx (m, d)) at the rows of X (emukit's IDifferentiable interface)."""
+        r = self.acquisition_gradients(X, 0.0, "min")
+        return r["dmu"], r["dvar"]
+
+    def grid_argmax(self, tables, best, task, cost_fix=1.0, cost_variable=False, refine=False):
+        """(max of EI / cost over the tensor grid, its coordinates (d,)): the per-set form of the batched sweep.
+        refine=True: the maximum refined off the grid inside the grid's box (SweepEngine.refine)."""
+        def result(session, out, g):
+            x = out.set_x[g] if refine and out.set_x[g] is not None else session.grid_point(g, out.set_indices[g])
+            return float(out.set_values[g]), np.asarray(x, np.float64)
         shared = self._shared()
         if shared is not None:
             session, g = shared
@@ -96,11 +124,9 @@ class SurrogateModel:
                 and float(cost_fix) == float(pr.cost_fix) and bool(cost_variable) == bool(pr.cost_variable)
             if same:
                 session.mark_interventional(g, self.X, self.Y)
-                out = session.best_per_set(best, task)
-                return float(out.set_values[g]), session.grid_point(g, out.set_indices[g])
+                return result(session, session.best_per_set(best, task, refine=refine), g)
         session = self._private_session(tables, cost_fix, cost_variable, with_grid=True)
-        out = session.best_per_set(best, task)
-        return float(out.set_values[0]), session.grid_point(0, out.set_indices[0])
+        return result(session, session.best_per_set(best, task, refine=refine), 0)
 
     def set_data(self, X, Y):
         """emukit GPyModelWrapper.set_data (reference call site Monitor.py:160)."""

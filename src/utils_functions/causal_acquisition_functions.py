@@ -2,7 +2,8 @@
 
 `evaluate(x)` keeps the reference signature, but the arithmetic -- posterior mean/variance at x, sd (u Phi(u) + phi(u))
 with u = (best - mu) / sd, sign flipped for task 'max' -- runs in the CUDA sweep kernel (csrc/sweep.cu) through
-`model.acquisition_points`.  Gradients are not provided: the grid argmax replaces L-BFGS (SURVEY.md §2 row 12)."""
+`model.acquisition_points`.  `evaluate_with_gradients(x)` differentiates the same quantity on the device
+(csrc/refine.cu, cbo_acq_grad) when the model provides gradients."""
 import numpy as np
 import scipy.stats
 
@@ -34,12 +35,18 @@ class CausalExpectedImprovement:
         out = self.model.acquisition_points(x, float(self.current_global_min) - float(self.jitter), self.task)
         return out["ei"].reshape(-1, 1)
 
+    def evaluate_with_gradients(self, x):
+        """(EI (m, 1), dEI/dx (m, d)) at the rows of x (reference :45-67)."""
+        x = np.atleast_2d(np.asarray(x, np.float64))
+        out = self.model.acquisition_gradients(x, float(self.current_global_min) - float(self.jitter), self.task)
+        return out["ei"].reshape(-1, 1), out["dei"].reshape(x.shape[0], -1)
+
     def __truediv__(self, cost):
         return _Quotient(self, cost)
 
     @property
     def has_gradients(self):
-        return False
+        return bool(getattr(self.model, "has_gradients", False))
 
 
 def get_standard_normal_pdf_cdf(x, mean, standard_deviation):

@@ -1,14 +1,16 @@
 """Acquisition maximiser (reference: src/utils_functions/causal_optimizer.py).  The reference draws
 `num_anchor_points` = 100 uniform anchors, keeps the best and refines it with L-BFGS (:19, :52-62); the build's
 deterministic replacement is the dense tensor-product grid with `num_anchor_points` points per dimension and the
-first argmax (SURVEY.md §0).  With a model that is backed by the CUDA sweep the whole search is one device pass."""
+first argmax (SURVEY.md §0).  With a model that is backed by the CUDA sweep the whole search is one device pass;
+`refine=True` then polishes the grid maximum off the grid with on-device gradients (the reference's L-BFGS step)."""
 import numpy as np
 
 
 class CausalGradientAcquisitionOptimizer:
-    def __init__(self, space, num_anchor_points=100):
+    def __init__(self, space, num_anchor_points=100, refine=False):
         self.space = space
         self.num_anchor_points = num_anchor_points
+        self.refine = refine
 
     def optimize(self, acquisition, context=None):
         """Returns (x (1, d), acquisition value there)."""
@@ -17,7 +19,8 @@ class CausalGradientAcquisitionOptimizer:
         model = getattr(ei, "model", None)
         if model is not None and hasattr(model, "grid_argmax"):
             fix, variable = cost.kernel_form() if cost is not None else (1.0, False)
-            value, x = model.grid_argmax(tables, float(ei.current_global_min) - float(ei.jitter), ei.task, fix, variable)
+            value, x = model.grid_argmax(tables, float(ei.current_global_min) - float(ei.jitter), ei.task, fix, variable,
+                                         refine=self.refine)
             return np.asarray(x, np.float64).reshape(1, -1), value
         # generic acquisition object: score the grid in chunks through its evaluate()
         mesh = np.meshgrid(*tables, indexing="ij")

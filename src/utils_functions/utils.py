@@ -17,12 +17,13 @@ def find_current_global(current_y, dict_interventions, task):
     return per_set[choose(per_set, key=per_set.get)]
 
 
-def find_next_y_point(space, model, current_global_best, evaluated_set, costs_functions, task="min"):
+def find_next_y_point(space, model, current_global_best, evaluated_set, costs_functions, task="min", refine=False):
     """Maximise EI / cost over the set's candidates and return (acquisition value (1,1), x_new (1,d)) (reference :29-37).
     The reference scores 100 random anchors and refines the best with L-BFGS; this build takes the argmax of the dense
-    tensor-product grid (100 points per dimension), evaluated by the CUDA sweep."""
+    tensor-product grid (100 points per dimension), evaluated by the CUDA sweep; refine=True refines that maximum off the
+    grid with on-device gradients."""
     cost_acquisition = Cost(costs_functions, evaluated_set)
-    optimizer = CausalGradientAcquisitionOptimizer(space)
+    optimizer = CausalGradientAcquisitionOptimizer(space, refine=refine)
     acquisition = CausalExpectedImprovement(current_global_best, task, model) / cost_acquisition
     x_new, y_acquisition = optimizer.optimize(acquisition)
     return np.asarray(y_acquisition, np.float64).reshape(1, 1), x_new
