@@ -8,7 +8,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CBO_B200_LIB") or os.path.join(HERE, "libcbo_b200.so")   # (the override is for kernel experiments)
 
-CBO_ABI_VERSION = 7
+CBO_ABI_VERSION = 8
 CBO_MAX_D = 4
 CBO_MAX_C = 8
 CBO_MAX_NINT = 128

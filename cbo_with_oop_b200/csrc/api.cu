@@ -70,7 +70,7 @@ int argmax_combine_impl(const cbo_set_best*, int, int, cbo_set_best*, cbo_sweep_
 size_t obs_gp_workspace_bytes_impl(const cbo_set_desc*, int);
 int obs_gp_fit_impl(const cbo_set_desc*, int, double, void*, size_t, int32_t*, cudaStream_t);
 int obs_gp_nll_impl(const cbo_set_desc*, void*, size_t, double*, cudaStream_t);
-int int_rows_table_impl(const cbo_set_desc&, cudaStream_t);
+int int_rows_table_impl(const cbo_set_desc&, const cbo_set_desc*, cudaStream_t);
 size_t refine_workspace_bytes_impl(const cbo_set_desc*, int);
 int acq_grad_impl(const cbo_set_desc*, const cbo_set_desc*, const double*, int, double, int, void*, size_t, cbo_acq_grad_out*, cudaStream_t);
 int refine_impl(const cbo_set_desc*, const cbo_set_desc*, int, double, int, const double*, int, double, void*, size_t, cbo_refine_result*,
@@ -126,11 +126,13 @@ int cbo_obs_gp_nll(const cbo_set_desc* h_set, void* d_workspace, size_t workspac
 
 int cbo_build_tables(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, void* stream) {
     if (int rc = validate_sets(h_sets, num_sets)) return rc;
+    CBO_REQUIRE(d_sets != nullptr, "cbo_build_tables: d_sets is NULL");
     return build_tables_impl(h_sets, d_sets, num_sets, (cudaStream_t)stream);
 }
 
 int cbo_prior_precompute(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, void* stream) {
     if (int rc = validate_sets(h_sets, num_sets)) return rc;
+    CBO_REQUIRE(d_sets != nullptr, "cbo_prior_precompute: d_sets is NULL");
     return prior_precompute_impl(h_sets, d_sets, num_sets, (cudaStream_t)stream);
 }
 
@@ -196,7 +198,7 @@ int cbo_refresh_trial(const cbo_set_desc* h_sets, cbo_set_desc* d_sets, int num_
         const cbo_set_desc* d = d_sets + refit_set;
         CBO_REQUIRE(!h->posterior_cached, "cbo_refresh_trial: the refitted set cannot be marked posterior_cached");
         if (computes_prior(*h)) {
-            if (int rc = int_rows_table_impl(*h, st)) return rc;
+            if (int rc = int_rows_table_impl(*h, d, st)) return rc;
             if (int rc = prior_eval_impl(h, d, 1, 1, d_workspace, workspace_bytes, st)) return rc;
         }
         if (int rc = posterior_fit_impl(h, d, 1, st)) return rc;

@@ -11,54 +11,19 @@
 
 namespace cbo {
 
+// Every table of every set in one launch: blockIdx.z = set * (CBO_MAX_D + 1) + table.  Table k < d is the grid table of
+// dimension k, table d is u_int.  A set with explicit points has no grid tables: its table 0 is tab[0] with one row per
+// point, formed like a row of u_int.  int_rows_only: blockIdx.z = set, and only the rows [int_row_begin, n_int) of u_int.
 __global__ void __launch_bounds__(256)
-table_kernel(const double* __restrict__ coords, int p, const double* __restrict__ xcol, int n_obs, int n_obs_pad,
-             double inv_l, double* __restrict__ out) {
+tables_kernel(const cbo_set_desc* __restrict__ sets, bool int_rows_only) {
+    const cbo_set_desc& S = sets[int_rows_only ? blockIdx.z : blockIdx.z / (CBO_MAX_D + 1)];
+    const int d = S.d, k = int_rows_only ? d : blockIdx.z % (CBO_MAX_D + 1);
+    if (!computes_prior(S) || k > d || (S.points && k > 0 && k < d)) return;
+    const int n_obs = S.n_obs, n_obs_pad = S.n_obs_pad;
     const int j = blockIdx.x * 256 + threadIdx.x;
     if (j >= n_obs_pad) return;
     const bool live = j < n_obs;
-    const double x = live ? xcol[j] : 0.0;
-    for (int i = blockIdx.y; i < p; i += gridDim.y) {
-        const double t = (coords[i] - x) * inv_l;
-        out[(size_t)i * n_obs_pad + j] = live ? exp(-0.5 * (t * t)) : 0.0;
-    }
-}
-
-__global__ void __launch_bounds__(256)
-points_table_kernel(const double* __restrict__ x_int, int n_int, int d, const double* __restrict__ x_obs_int, int n_obs,
-                    int n_obs_pad, double il0, double il1, double il2, double il3, double* __restrict__ out) {
-    const int j = blockIdx.x * 256 + threadIdx.x;
-    if (j >= n_obs_pad) return;
-    const bool live = j < n_obs;
-    const double il[CBO_MAX_D] = {il0, il1, il2, il3};
-    double x[CBO_MAX_D];
-#pragma unroll
-    for (int k = 0; k < CBO_MAX_D; ++k) x[k] = (live && k < d) ? x_obs_int[(size_t)k * n_obs + j] : 0.0;
-    for (int i = blockIdx.y; i < n_int; i += gridDim.y) {
-        double r2 = 0.0;
-#pragma unroll
-        for (int k = 0; k < CBO_MAX_D; ++k) {
-            if (k < d) {
-                const double t = (x_int[i * d + k] - x[k]) * il[k];
-                r2 += t * t;
-            }
-        }
-        out[(size_t)i * n_obs_pad + j] = live ? exp(-0.5 * r2) : 0.0;
-    }
-}
-
-// Every table of every set in one launch (needs the descriptors on the device): blockIdx.z = set * (CBO_MAX_D + 1) + table,
-// table == d being the interventional-row table u_int.  Explicit-point sets keep their own launch.
-__global__ void __launch_bounds__(256)
-tables_batched_kernel(const cbo_set_desc* __restrict__ sets) {
-    const cbo_set_desc& S = sets[blockIdx.z / (CBO_MAX_D + 1)];
-    const int k = blockIdx.z % (CBO_MAX_D + 1);
-    if (!computes_prior(S) || S.points || k > S.d) return;
-    const int n_obs = S.n_obs, n_obs_pad = S.n_obs_pad, d = S.d;
-    const int j = blockIdx.x * 256 + threadIdx.x;
-    if (j >= n_obs_pad) return;
-    const bool live = j < n_obs;
-    if (k < d) {
+    if (k < d && !S.points) {
         const double x = live ? S.x_obs_int[(size_t)k * n_obs + j] : 0.0, inv_l = 1.0 / S.ls_int[k];
         const double* __restrict__ coords = S.grid[k];
         double* __restrict__ out = S.tab[k];
@@ -66,95 +31,68 @@ tables_batched_kernel(const cbo_set_desc* __restrict__ sets) {
             const double t = (coords[i] - x) * inv_l;
             out[(size_t)i * n_obs_pad + j] = live ? exp(-0.5 * (t * t)) : 0.0;
         }
-    } else {
-        double x[CBO_MAX_D], il[CBO_MAX_D];
+        return;
+    }
+    // rows of d coordinates: the explicit points (table 0) or the interventional rows (table d)
+    const bool points = k < d;
+    const double* __restrict__ src = points ? S.points : S.x_int;
+    double* __restrict__ out = points ? S.tab[0] : S.u_int;
+    const int r0 = int_rows_only ? S.int_row_begin : 0, rows = points ? (int)S.g_total : S.n_int;
+    double x[CBO_MAX_D], il[CBO_MAX_D];
+#pragma unroll
+    for (int q = 0; q < CBO_MAX_D; ++q) {
+        x[q] = (live && q < d) ? S.x_obs_int[(size_t)q * n_obs + j] : 0.0;
+        il[q] = q < d ? 1.0 / S.ls_int[q] : 0.0;
+    }
+    for (int i = r0 + blockIdx.y; i < rows; i += gridDim.y) {
+        double r2 = 0.0;
 #pragma unroll
         for (int q = 0; q < CBO_MAX_D; ++q) {
-            x[q] = (live && q < d) ? S.x_obs_int[(size_t)q * n_obs + j] : 0.0;
-            il[q] = q < d ? 1.0 / S.ls_int[q] : 0.0;
-        }
-        for (int i = blockIdx.y; i < S.n_int; i += gridDim.y) {
-            double r2 = 0.0;
-#pragma unroll
-            for (int q = 0; q < CBO_MAX_D; ++q) {
-                if (q < d) {
-                    const double t = (S.x_int[i * d + q] - x[q]) * il[q];
-                    r2 += t * t;
-                }
+            if (q < d) {
+                const double t = (src[i * d + q] - x[q]) * il[q];
+                r2 += t * t;
             }
-            S.u_int[(size_t)i * n_obs_pad + j] = live ? exp(-0.5 * r2) : 0.0;
         }
+        out[(size_t)i * n_obs_pad + j] = live ? exp(-0.5 * r2) : 0.0;
     }
 }
 
-// The interventional-row table of ONE set, rows [int_row_begin, n_int) only (a post-intervention trial appends one row; the
-// grid tables do not depend on x_int).
-int int_rows_table_impl(const cbo_set_desc& S, cudaStream_t st) {
+static unsigned row_blocks(int rows) { return (unsigned)(rows < 1024 ? rows : 1024); }
+
+// The interventional-row table of the refitted set of a post-intervention trial, rows [int_row_begin, n_int) only (the grid
+// tables do not depend on x_int).  `d_set`: the set's descriptor on the device.
+int int_rows_table_impl(const cbo_set_desc& S, const cbo_set_desc* d_set, cudaStream_t st) {
     if (!computes_prior(S) || S.int_row_begin >= S.n_int) return 0;
     CBO_REQUIRE(S.u_int && S.x_int && S.x_obs_int, "cbo_refresh_trial: NULL u_int/x_int/x_obs_int pointer");
-    const int r0 = S.int_row_begin, rows = S.n_int - r0;
-    const double il[CBO_MAX_D] = {1.0 / S.ls_int[0], S.d > 1 ? 1.0 / S.ls_int[1] : 0.0, S.d > 2 ? 1.0 / S.ls_int[2] : 0.0,
-                                  S.d > 3 ? 1.0 / S.ls_int[3] : 0.0};
-    points_table_kernel<<<dim3((S.n_obs_pad + 255) / 256, (unsigned)(rows < 1024 ? rows : 1024)), 256, 0, st>>>(
-        S.x_int + (size_t)r0 * S.d, rows, S.d, S.x_obs_int, S.n_obs, S.n_obs_pad, il[0], il[1], il[2], il[3],
-        S.u_int + (size_t)r0 * S.n_obs_pad);
+    tables_kernel<<<dim3((S.n_obs_pad + 255) / 256, row_blocks(S.n_int - S.int_row_begin)), 256, 0, st>>>(d_set, true);
     note_launch();
     CBO_CUDA(cudaGetLastError());
     return 0;
 }
 
 int build_tables_impl(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, cudaStream_t st) {
-    bool batched = d_sets != nullptr && num_sets > 1 && num_sets * (CBO_MAX_D + 1) <= 65535;
-    if (batched) {
-        int npad_max = 0, rows_max = 1;
-        for (int s = 0; s < num_sets; ++s) {
-            const cbo_set_desc& S = h_sets[s];
-            if (!computes_prior(S) || S.points) continue;
-            for (int k = 0; k < S.d; ++k) {
-                CBO_REQUIRE(S.tab[k] && S.grid[k] && S.x_obs_int, "cbo_build_tables: set %d has a NULL table/grid pointer", s);
-                if (S.p[k] > rows_max) rows_max = S.p[k];
-            }
-            CBO_REQUIRE(S.u_int && S.x_int, "cbo_build_tables: set %d has a NULL u_int/x_int pointer", s);
-            if (S.n_int > rows_max) rows_max = S.n_int;
-            if (S.n_obs_pad > npad_max) npad_max = S.n_obs_pad;
-        }
-        if (npad_max > 0) {
-            tables_batched_kernel<<<dim3((unsigned)((npad_max + 255) / 256), (unsigned)(rows_max < 256 ? rows_max : 256),
-                                         (unsigned)(num_sets * (CBO_MAX_D + 1))), 256, 0, st>>>(d_sets);
-            note_launch();
-            CBO_CUDA(cudaGetLastError());
-        }
-    }
+    int npad_max = 0, rows_max = 1;
     for (int s = 0; s < num_sets; ++s) {
         const cbo_set_desc& S = h_sets[s];
-        if (!computes_prior(S) || (batched && !S.points)) continue;
-        const unsigned gx = (S.n_obs_pad + 255) / 256;
-        const double il[CBO_MAX_D] = {1.0 / S.ls_int[0], S.d > 1 ? 1.0 / S.ls_int[1] : 0.0, S.d > 2 ? 1.0 / S.ls_int[2] : 0.0,
-                                      S.d > 3 ? 1.0 / S.ls_int[3] : 0.0};
-        if (S.points) {  // explicit candidates: one table with a row per candidate
+        if (!computes_prior(S)) continue;
+        if (S.points) {
             CBO_REQUIRE(S.tab[0] && S.x_obs_int, "cbo_build_tables: set %d has a NULL table pointer", s);
             CBO_REQUIRE(S.g_total < 2147483647LL / CBO_MAX_D, "cbo_build_tables: set %d has too many explicit points", s);
-            if (S.g_total > 0) {
-                const unsigned gy = (unsigned)(S.g_total < 1024 ? S.g_total : 1024);
-                points_table_kernel<<<dim3(gx, gy), 256, 0, st>>>(S.points, (int)S.g_total, S.d, S.x_obs_int, S.n_obs, S.n_obs_pad,
-                                                                  il[0], il[1], il[2], il[3], S.tab[0]);
-                note_launch();
-            }
+            if (S.g_total > rows_max) rows_max = (int)S.g_total;
         }
         for (int k = 0; k < (S.points ? 0 : S.d); ++k) {
             CBO_REQUIRE(S.tab[k] && S.grid[k] && S.x_obs_int, "cbo_build_tables: set %d has a NULL table/grid pointer", s);
-            const unsigned gy = (unsigned)(S.p[k] < 1024 ? S.p[k] : 1024);
-            table_kernel<<<dim3(gx, gy), 256, 0, st>>>(S.grid[k], S.p[k], S.x_obs_int + (size_t)k * S.n_obs, S.n_obs,
-                                                       S.n_obs_pad, 1.0 / S.ls_int[k], S.tab[k]);
-            note_launch();
+            if (S.p[k] > rows_max) rows_max = S.p[k];
         }
         CBO_REQUIRE(S.u_int && S.x_int, "cbo_build_tables: set %d has a NULL u_int/x_int pointer", s);
-        const unsigned gy = (unsigned)(S.n_int < 1024 ? S.n_int : 1024);
-        points_table_kernel<<<dim3(gx, gy), 256, 0, st>>>(S.x_int, S.n_int, S.d, S.x_obs_int, S.n_obs, S.n_obs_pad, il[0], il[1],
-                                                          il[2], il[3], S.u_int);
-        note_launch();
-        CBO_CUDA(cudaGetLastError());
+        if (S.n_int > rows_max) rows_max = S.n_int;
+        if (S.n_obs_pad > npad_max) npad_max = S.n_obs_pad;
     }
+    if (npad_max == 0) return 0;
+    // num_sets <= 4096 (validate_sets): the grid's z extent stays within 65535
+    tables_kernel<<<dim3((npad_max + 255) / 256, row_blocks(rows_max), num_sets * (CBO_MAX_D + 1)), 256, 0, st>>>(d_sets, false);
+    note_launch();
+    CBO_CUDA(cudaGetLastError());
     return 0;
 }
 

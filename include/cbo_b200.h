@@ -30,7 +30,7 @@ extern "C" {
 #define CBO_API
 #endif
 
-#define CBO_ABI_VERSION 7
+#define CBO_ABI_VERSION 8
 #define CBO_MAX_D 4          /* intervened dimensions per exploration set (reference uses 1..3) */
 #define CBO_MAX_C 8          /* conditioning dimensions of an observational GP */
 #define CBO_MAX_NINT 128     /* interventional rows per set (reference: 10 .. ~50) */
@@ -158,14 +158,15 @@ CBO_API int cbo_obs_gp_nll(const cbo_set_desc* h_set, void* d_workspace, size_t 
 /* K0. exp tables: tab[k][i][j] = exp(-.5 ((grid[k][i] - x_obs_int[k][j]) / ls_int[k])^2) and
  * u_int[i][j] = exp(-.5 sum_k ((x_int[i][k] - x_obs_int[k][j]) / ls_int[k])^2).
  * Replaces the kernel evaluations inside gp.predict at DoCalculus.py:77 for the intervened columns.
- * `d_sets` may be NULL; with the descriptors on the device every table of every set is written by ONE launch. */
+ * `d_sets` (required) is read by the kernel: every table of every set is written by ONE launch. */
 CBO_API int cbo_build_tables(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, void* stream);
 
 /* K1a. P, pbar, w, M from the observational GP state and the conditioning samples.
  * Replaces the per-candidate np.hstack + gp.predict set-up of DoCalculus.py:68-89 (done once per
  * observation instead of once per candidate; SURVEY.md App. A.5).
- * `d_sets` may be NULL; with the descriptors on the device and a P buffer per set (no two sets sharing one) all sets
- * go through one launch per stage instead of two launches per set. */
+ * `d_sets` (required) is read by the kernels.  Sets without conditioning columns share one launch.  The others run two
+ * stages, P then M; consecutive sets share one launch per stage unless a set's P overlaps another set's (such sets run
+ * one after the other) or its N is large enough to fill the GPU on its own (then it runs alone, on the TMA pipeline). */
 CBO_API int cbo_prior_precompute(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, void* stream);
 
 /* K1b. causal prior m(x) = u.w, v(x) = s2 + noise - u^T M u.

@@ -69,6 +69,20 @@ def test_argument_validation_reports_through_last_error(lib):
         _lib.check(-1, "demo")
 
 
+def test_tables_and_prior_precompute_refuse_host_only_descriptors(lib):
+    """Both stages read every set from the device copy of the descriptors: a NULL d_sets is refused, with a message,
+    after the descriptors themselves have passed validation."""
+    from cbo_with_oop_b200 import _lib
+    h = (_lib.SetDesc * 1)()
+    h[0].d, h[0].n_int, h[0].p[0], h[0].g_total, h[0].g_count, h[0].cost_fix = 1, 5, 10, 10, 10, 1.0
+    h[0].causal, h[0].n_obs, h[0].n_obs_pad, h[0].ls_int[0] = 1, 100, 128, 1.0
+    assert lib.cbo_sweep(h, None, 1, 0.0, 1, None, None, None, None) == -1
+    assert lib.cbo_last_error() == b"cbo_sweep: d_sets is NULL"      # validate_sets accepted the descriptor
+    for fn in (lib.cbo_build_tables, lib.cbo_prior_precompute):
+        assert fn(h, None, 1, None) == -1
+        assert b"d_sets" in lib.cbo_last_error()
+
+
 def test_no_cpu_fallback(monkeypatch):
     """Without a CUDA device the engine refuses to start (the product path is the CUDA library).  On a machine with a
     GPU the device is hidden from the engine."""
