@@ -8,7 +8,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CBO_B200_LIB") or os.path.join(HERE, "libcbo_b200.so")   # (the override is for kernel experiments)
 
-CBO_ABI_VERSION = 8
+CBO_ABI_VERSION = 9
 CBO_MAX_D = 4
 CBO_MAX_C = 8
 CBO_MAX_NINT = 128
@@ -37,7 +37,7 @@ class SetDesc(C.Structure):
         ("cost_fix", C.c_double), ("cost_variable", C.c_int32), ("prior_external", C.c_int32),
         ("m", _dp), ("v", _dp), ("mu", _dp), ("var", _dp), ("ei", _dp), ("acq", _dp),
         ("posterior_cached", C.c_int32), ("int_row_begin", C.c_int32), ("y_obs", C.c_void_p),
-        ("points", _dp),
+        ("points", _dp), ("hyper", _dp),
     ]
 
 
@@ -61,6 +61,15 @@ class RefineResult(C.Structure):
                 ("iterations", C.c_int32), ("status", C.c_int32)]
 
 
+class HyperResult(C.Structure):
+    """Mirror of cbo_hyper_result (one exploration set's marginal-likelihood fit)."""
+    _fields_ = [("variance", C.c_double), ("lengthscale", C.c_double), ("nll", C.c_double), ("nll_start", C.c_double),
+                ("iterations", C.c_int32), ("status", C.c_int32), ("start", C.c_int32), ("jitter_tries", C.c_int32)]
+
+
+CBO_HYPER_STARTS = 9
+HYPER_STATUS = {0: "converged", 1: "max_iter", 2: "line_search_failed", 3: "not_positive_definite"}
+
 REFINE_STATUS = {0: "converged", 1: "max_iter", 2: "line_search_failed", 3: "skipped_external_prior",
                  4: "skipped_explicit_points", 5: "skipped_nonfinite"}
 
@@ -71,7 +80,7 @@ EXPORTS = [
     "cbo_obs_gp_fit", "cbo_obs_gp_nll",
     "cbo_build_tables", "cbo_prior_precompute", "cbo_prior_eval", "cbo_posterior_fit", "cbo_sweep",
     "cbo_argmax_combine", "cbo_sem_eval", "cbo_refresh_trial", "cbo_acq_grad", "cbo_refine",
-    "cbo_refine_workspace_bytes",
+    "cbo_refine_workspace_bytes", "cbo_posterior_nll", "cbo_posterior_hyper_fit", "cbo_posterior_hyper_workspace_bytes",
 ]
 CBO_SEM_MAX_NODES, CBO_SEM_MAX_TERMS, CBO_SEM_BLOCKS = 16, 96, 64
 SEM_FUNCS = {"id": 0, "exp": 1, "cos": 2, "sin": 3, "square": 4}
@@ -140,6 +149,11 @@ def load() -> C.CDLL:
                                C.c_size_t, C.c_void_p, C.c_void_p]
     for name in EXPORTS[10:]:
         getattr(lib, name).restype = C.c_int
+    lib.cbo_posterior_nll.argtypes = [P, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+    lib.cbo_posterior_hyper_fit.argtypes = [P, C.c_void_p, C.c_int, C.POINTER(C.c_double), C.c_int, C.c_double, C.c_void_p,
+                                            C.c_size_t, C.c_void_p, C.c_void_p]
+    lib.cbo_posterior_hyper_workspace_bytes.restype = C.c_size_t
+    lib.cbo_posterior_hyper_workspace_bytes.argtypes = [P, C.c_int]
     lib.cbo_refine_workspace_bytes.restype = C.c_size_t
     lib.cbo_refine_workspace_bytes.argtypes = [P, C.c_int]
     if lib.cbo_abi_version() != CBO_ABI_VERSION:

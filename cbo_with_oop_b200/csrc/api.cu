@@ -75,6 +75,10 @@ size_t refine_workspace_bytes_impl(const cbo_set_desc*, int);
 int acq_grad_impl(const cbo_set_desc*, const cbo_set_desc*, const double*, int, double, int, void*, size_t, cbo_acq_grad_out*, cudaStream_t);
 int refine_impl(const cbo_set_desc*, const cbo_set_desc*, int, double, int, const double*, int, double, void*, size_t, cbo_refine_result*,
                 cudaStream_t);
+int posterior_nll_impl(const cbo_set_desc*, const cbo_set_desc*, int, double*, cudaStream_t);
+size_t hyper_workspace_bytes_impl(int);
+int hyper_fit_impl(const cbo_set_desc*, const cbo_set_desc*, int, const double*, int, double, void*, size_t, cbo_hyper_result*,
+                   cudaStream_t);
 int sem_eval_impl(const cbo_sem_node*, int, const cbo_sem_term*, int, const double*, int, long long, const int32_t*, const double*, int,
                   int, double*, double*, cudaStream_t);
 
@@ -95,7 +99,7 @@ long cbo_offsetof_set_desc(const char* field) {
     F(d) F(c) F(n_obs) F(n_obs_pad) F(n_mc) F(n_mc_pad) F(n_int) F(causal) F(p) F(g_total) F(g_begin) F(g_count)
     F(x_obs_int) F(x_obs_cond) F(mc_cond) F(alpha_obs) F(kyinv) F(ls_int) F(ls_cond) F(s2) F(noise)
     F(tab) F(u_int) F(P) F(pbar) F(w) F(M) F(grid) F(x_int) F(y_int) F(m_int) F(v_int) F(L) F(alpha) F(sqrt_v_int)
-    F(fit_info) F(cost_fix) F(cost_variable) F(prior_external) F(m) F(v) F(mu) F(var) F(ei) F(acq) F(posterior_cached) F(int_row_begin) F(y_obs) F(points)
+    F(fit_info) F(cost_fix) F(cost_variable) F(prior_external) F(m) F(v) F(mu) F(var) F(ei) F(acq) F(posterior_cached) F(int_row_begin) F(y_obs) F(points) F(hyper)
 #undef F
     return -1;
 }
@@ -228,6 +232,25 @@ int cbo_refine(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_s
     if (int rc = validate_sets(h_sets, num_sets)) return rc;
     return refine_impl(h_sets, d_sets, num_sets, best, task_sign, d_x0, max_iter, gtol, d_workspace, workspace_bytes, d_out,
                        (cudaStream_t)stream);
+}
+
+int cbo_posterior_nll(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, double* d_out, void* stream) {
+    if (int rc = validate_sets(h_sets, num_sets)) return rc;
+    CBO_REQUIRE(d_sets != nullptr, "cbo_posterior_nll: d_sets is NULL");
+    CBO_REQUIRE(d_out != nullptr, "cbo_posterior_nll: d_out is NULL");
+    return posterior_nll_impl(h_sets, d_sets, num_sets, d_out, (cudaStream_t)stream);
+}
+
+size_t cbo_posterior_hyper_workspace_bytes(const cbo_set_desc* h_sets, int num_sets) {
+    if (!h_sets || num_sets < 1) return 0;
+    return hyper_workspace_bytes_impl(num_sets);
+}
+
+int cbo_posterior_hyper_fit(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, const double* h_bounds, int max_iter,
+                            double gtol, void* d_workspace, size_t workspace_bytes, cbo_hyper_result* d_out, void* stream) {
+    if (int rc = validate_sets(h_sets, num_sets)) return rc;
+    CBO_REQUIRE(d_sets != nullptr, "cbo_posterior_hyper_fit: d_sets is NULL");
+    return hyper_fit_impl(h_sets, d_sets, num_sets, h_bounds, max_iter, gtol, d_workspace, workspace_bytes, d_out, (cudaStream_t)stream);
 }
 
 int cbo_sem_eval(const cbo_sem_node* d_nodes, int num_nodes, const cbo_sem_term* d_terms, int num_terms, const double* d_noise,

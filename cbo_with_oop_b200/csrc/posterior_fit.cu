@@ -2,9 +2,10 @@
 // shared memory.
 //
 // Replaces GPRegression(...) at GaussianProcessFactory.py:57-73, i.e. GPy's ExactGaussianInference:
-//   causal     : K = exp(-.5 r^2) + sqrt(v(X)) sqrt(v(X))^T   (CausalRBF.K, causal_kernels.py:45-62; l = 1, s2 = 1)
+//   causal     : K = s2 exp(-.5 r^2 / l^2) + sqrt(v(X)) sqrt(v(X))^T   (CausalRBF.K, causal_kernels.py:45-62)
 //                resid = y - m(X)                              (Mapping.f = mean function, :65-68)
-//   non-causal : K = exp(-.5 r^2), resid = y                   (:57-60)
+//   non-causal : K = s2 exp(-.5 r^2 / l^2), resid = y          (:57-60)
+//   (s2, l) = hyper[0..1], or the reference's (1, 1) when `hyper` is NULL (the scaling by 1 is exact: same bits)
 //   Ky = K + (1e-10 + 1e-8) I ; L = jitchol(Ky) ; alpha = Ky^-1 resid
 // Output `L`: the factor in the lower triangle; for n <= 48 the strict upper triangle carries L^-T (for K3), else zeros.
 // jitchol rule (GPy util.linalg): plain Cholesky first; on a non-positive pivot retry with
@@ -31,6 +32,7 @@ posterior_fit_kernel(const cbo_set_desc* __restrict__ sets) {
     double* dsq = rinv + n;                           // L_ii
     bool failed = false;
     __shared__ double diag_mean;
+    const double s2 = S.hyper ? S.hyper[0] : 1.0, il = S.hyper ? 1.0 / S.hyper[1] : 1.0;
 
     for (int i = tid; i < n; i += kFitThreads) {
         sv[i] = S.causal ? sqrt(S.v_int[i]) : 0.0;
@@ -47,10 +49,10 @@ posterior_fit_kernel(const cbo_set_desc* __restrict__ sets) {
             const int i = e / n, j = e % n;
             double r2 = 0.0;
             for (int k = 0; k < d; ++k) {
-                const double t = xs[i * d + k] - xs[j * d + k];
+                const double t = (xs[i * d + k] - xs[j * d + k]) * il;
                 r2 += t * t;
             }
-            double kij = exp(-0.5 * r2) + sv[i] * sv[j];
+            double kij = fma(sv[i], sv[j], __dmul_rn(s2, exp(-0.5 * r2)));
             if (i == j) kij += (1e-10 + 1e-8) + jitter;
             A[e] = kij;
         }

@@ -8,9 +8,9 @@
 //   causal prior    u_j = prod_k exp(-.5 ((x_k - X_kj) / l_k)^2),  m = u.w,  v = s2 + noise - u^T M u
 //                   a_kj = u_j (x_k - X_kj) / l_k^2,  dm/dx_k = -sum_j a_kj w_j,  dv/dx_k = 2 a_k^T M u
 //                   (each sum is accumulated with the weights a_kj themselves: no x_k u^T M u - sum_j X_kj ... cancellation)
-//   per-set GP      e_i = exp(-.5 |x - x_i|^2),  k*_i = e_i + sv_i sqrt(v) (non-causal: e_i, m = v = 0)
-//                   dk*_i = -e_i (x - x_i) + sv_i dv / (2 sqrt v)
-//                   mu = m + k*.alpha,  var = (1 + v) - |L^-1 k*|^2 + 1e-10   (as K3 computes them)
+//   per-set GP      e_i = s2 exp(-.5 |x - x_i|^2 / l^2),  k*_i = e_i + sv_i sqrt(v) (non-causal: e_i, m = v = 0)
+//                   dk*_i = -e_i (x - x_i) / l^2 + sv_i dv / (2 sqrt v)     ((s2, l) = hyper, (1, 1) when NULL)
+//                   mu = m + k*.alpha,  var = (s2 + v) - |L^-1 k*|^2 + 1e-10   (as K3 computes them)
 //                   dmu = dm + sum_i alpha_i dk*_i,  dvar = dv - 2 beta^T dk*,  beta = L^-T L^-1 k*
 //   acquisition     u = (best - mu) / sd,  ei = sign sd (u Phi + phi),  dei = -sign Phi dmu + sign phi dvar / (2 sd)
 //                   c = cost_fix + cost_variable sum |x_k|,  acq = ei / c,  dacq = (dei - acq dc) / c
@@ -239,7 +239,8 @@ struct RefSmem {
     double* Lp;     // packed lower triangle of L, row i at i (i + 1) / 2
     double* al;     // alpha
     double* sv;     // sqrt(v_int) (0 for a non-causal set)
-    double* xs;     // x_int, n x d
+    double* xs;     // x_int / l, n x d
+    double s2, il;  // per-set GP variance and 1 / lengthscale
 };
 inline size_t ref_smem_bytes(int n) { return ((size_t)n * (n + 1) / 2 + 2 * (size_t)n + (size_t)n * CBO_MAX_D) * sizeof(double); }
 
@@ -249,6 +250,8 @@ __device__ void stage_posterior(const cbo_set_desc& S, RefSmem& sm, double* base
     sm.al = sm.Lp + (size_t)n * (n + 1) / 2;
     sm.sv = sm.al + n;
     sm.xs = sm.sv + n;
+    sm.s2 = S.hyper ? S.hyper[0] : 1.0;
+    sm.il = S.hyper ? 1.0 / S.hyper[1] : 1.0;
     for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
         const int i = e / n, j = e % n;
         if (j <= i) sm.Lp[i * (i + 1) / 2 + j] = S.L[e];
@@ -257,7 +260,7 @@ __device__ void stage_posterior(const cbo_set_desc& S, RefSmem& sm, double* base
         sm.al[i] = S.alpha[i];
         sm.sv[i] = S.causal ? S.sqrt_v_int[i] : 0.0;
     }
-    for (int i = threadIdx.x; i < n * d; i += blockDim.x) sm.xs[i] = S.x_int[i];
+    for (int i = threadIdx.x; i < n * d; i += blockDim.x) sm.xs[i] = S.x_int[i] * sm.il;
 }
 
 // partials: the set's slots of this point's batch (NULL when the set has no device prior); q = point within the batch
@@ -295,6 +298,9 @@ __device__ void eval_point(const cbo_set_desc& S, const RefSmem& sm, const doubl
     // rows i = lane + 32 r of k*, dk*
     double ks[4], dks[4][CBO_MAX_D], rr[4];
     double mu_p = 0.0, dmu_p[CBO_MAX_D] = {0.0, 0.0, 0.0, 0.0};
+    double xl[CBO_MAX_D];
+#pragma unroll
+    for (int k = 0; k < CBO_MAX_D; ++k) xl[k] = x[k] * sm.il;
 #pragma unroll
     for (int r = 0; r < 4; ++r) {
         const int i = lane + 32 * r;
@@ -305,13 +311,13 @@ __device__ void eval_point(const cbo_set_desc& S, const RefSmem& sm, const doubl
             double r2 = 0.0, z[CBO_MAX_D];
 #pragma unroll
             for (int k = 0; k < CBO_MAX_D; ++k) {
-                z[k] = k < d ? x[k] - sm.xs[i * d + k] : 0.0;
+                z[k] = k < d ? xl[k] - sm.xs[i * d + k] : 0.0;
                 r2 = fma(z[k], z[k], r2);
             }
-            const double e = exp(-0.5 * r2);
-            ks[r] = e + sm.sv[i] * sqv;
+            const double e = __dmul_rn(sm.s2, exp(-0.5 * r2));
+            ks[r] = fma(sm.sv[i], sqv, e);
 #pragma unroll
-            for (int k = 0; k < CBO_MAX_D; ++k) dks[r][k] = fma(-e, z[k], sm.sv[i] * dv[k] * hv);
+            for (int k = 0; k < CBO_MAX_D; ++k) dks[r][k] = fma(-e, __dmul_rn(z[k], sm.il), sm.sv[i] * dv[k] * hv);
             mu_p = fma(ks[r], sm.al[i], mu_p);
 #pragma unroll
             for (int k = 0; k < CBO_MAX_D; ++k) dmu_p[k] = fma(sm.al[i], dks[r][k], dmu_p[k]);
@@ -342,7 +348,7 @@ __device__ void eval_point(const cbo_set_desc& S, const RefSmem& sm, const doubl
 #pragma unroll
     for (int r = 0; r < 4; ++r) ss = fma(rr[r], rr[r], ss);
     ss = warp_sum(ss);
-    const double var = ((1.0 + v) - ss) + 1e-10;
+    const double var = ((sm.s2 + v) - ss) + 1e-10;
     // beta = L^-T t (backward substitution; lane j % 32 owns beta_j)
 #pragma unroll
     for (int rb = 3; rb >= 0; --rb) {

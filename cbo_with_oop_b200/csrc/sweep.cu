@@ -1,9 +1,12 @@
 // K3 + K4 -- posterior predict, Expected Improvement / cost and the first-argmax over every candidate.
 //
 // Per candidate x of set s (one thread each; L, alpha, X_I staged once per CTA in shared memory):
-//   k*_i = exp(-.5 |x - X_I,i|^2) + sqrt(v_I,i) sqrt(v(x))        CausalRBF.K(X_I, x), causal_kernels.py:55-62
+//   k*_i = s2 exp(-.5 |x - X_I,i|^2 / l^2) + sqrt(v_I,i) sqrt(v(x))   CausalRBF.K(X_I, x), causal_kernels.py:55-62
 //   mu   = m(x) + k*.alpha                                           GPy PosteriorExact._raw_predict + mean function
-//   t    = L^-1 k* ; var = (1 + v(x)) - |t|^2 + 1e-10                Kdiag :64-79, dtrtrs, Gaussian noise
+//   t    = L^-1 k* ; var = (s2 + v(x)) - |t|^2 + 1e-10               Kdiag :64-79, dtrtrs, Gaussian noise
+//   (s2, l) = cbo_set_desc.hyper, (1, 1) when NULL.  1 / l scales the staged coordinates (x_int, the candidate, the
+//   differences behind the separable tables) once, s2 is folded into the leading-dimension table and the A fragments: the
+//   per-candidate arithmetic is unchanged, and at (1, 1) every product is by 1.0, so the results are those of l = s2 = 1.
 //          (forward substitution for n <= 16 and n > 48; a DMMA product with L^-1 for 16 < n <= 48: sweep_mma_kernel)
 //   EI   = sd (u Phi(u) + phi(u)), u = (best - mu) / sd, negated for task 'max'   causal_acquisition_functions.py:33-43,85-87
 //   acq  = EI / cost(x)                                              utils.py:34, cost_functions.py:11-17
@@ -34,7 +37,7 @@ struct SweepSmem {
 // (fully unrolled, one broadcast LDS per FMA); NREG == 0: any n <= CBO_MAX_NINT, the vector lives in a shared-memory
 // column owned by the thread.
 template <int NREG>
-__device__ __forceinline__ void posterior_at(const SweepSmem& sm, int n, int d, const double (&x)[CBO_MAX_D], double svg,
+__device__ __forceinline__ void posterior_at(const SweepSmem& sm, int n, int d, const double (&x)[CBO_MAX_D], double svg, double s2,
                                              int tid, double& mu, double& ss) {
     mu = 0.0; ss = 0.0;
     if constexpr (NREG > 0) {
@@ -47,7 +50,7 @@ __device__ __forceinline__ void posterior_at(const SweepSmem& sm, int n, int d, 
                 for (int k = 0; k < CBO_MAX_D; ++k) {
                     if (k < d) { const double q = x[k] - sm.xs[i * d + k]; r2 = fma(q, q, r2); }
                 }
-                const double ks = exp(-0.5 * r2) + sm.sv[i] * svg;
+                const double ks = fma(sm.sv[i], svg, __dmul_rn(s2, exp(-0.5 * r2)));
                 mu = fma(ks, sm.al[i], mu);
                 const double* __restrict__ Li = sm.Lp + i * (i + 1) / 2;
                 // four interleaved partial sums: the row's dot product is a dependent FMA chain, and with 3-5 CTAs per SM
@@ -71,7 +74,7 @@ __device__ __forceinline__ void posterior_at(const SweepSmem& sm, int n, int d, 
             for (int k = 0; k < CBO_MAX_D; ++k) {
                 if (k < d) { const double q = x[k] - sm.xs[i * d + k]; r2 = fma(q, q, r2); }
             }
-            const double ks = exp(-0.5 * r2) + sm.sv[i] * svg;
+            const double ks = fma(sm.sv[i], svg, __dmul_rn(s2, exp(-0.5 * r2)));
             mu = fma(ks, sm.al[i], mu);
             const double* __restrict__ Li = sm.Lp + i * (i + 1) / 2;
             double a = ks;
@@ -151,6 +154,7 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
     const int n = S.n_int, d = S.d, tid = threadIdx.x;
     const bool causal = S.causal != 0;
     const bool cached = S.posterior_cached != 0;   // mu / var of an earlier sweep are still valid: EI refresh only
+    const double s2 = S.hyper ? S.hyper[0] : 1.0, il = S.hyper ? 1.0 / S.hyper[1] : 1.0;
     if (sweep_class(S) != (NREG == 0 ? kClsGeneric : (SEP ? kClsFmaSep : kClsFma))) return;       // another launch's set
     const bool sep = SEP;
     const int p_last = S.points ? 1 : S.p[d - 1];
@@ -183,12 +187,12 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
             sm.al[i] = S.alpha[i];
             sm.sv[i] = causal ? S.sqrt_v_int[i] : 0.0;
         }
-        for (int i = tid; i < n * d; i += kSweepThreads) sm.xs[i] = S.x_int[i];
+        for (int i = tid; i < n * d; i += kSweepThreads) sm.xs[i] = S.x_int[i] * il;
         if (sep) {
             const double* __restrict__ gl = S.grid[d - 1];
             for (int e = tid; e < n * p_last; e += kSweepThreads) {
                 const int i = e / p_last, j = e - i * p_last;
-                const double q = gl[j] - S.x_int[i * d + d - 1];
+                const double q = (gl[j] - S.x_int[i * d + d - 1]) * il;
                 eLast[i * ldl + j] = exp(-0.5 * (q * q));
             }
             const long long last_row = (gidx0 + cnt - 1) / p_last;
@@ -199,11 +203,11 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
                 double r2 = 0.0;
                 for (int k = d - 2; k >= 0; --k) {
                     const long long pk = S.p[k];
-                    const double q = S.grid[k][(int)(rr % pk)] - S.x_int[i * d + k];
+                    const double q = (S.grid[k][(int)(rr % pk)] - S.x_int[i * d + k]) * il;
                     r2 = fma(q, q, r2);
                     rr /= pk;
                 }
-                eLead[i * ldr + r] = exp(-0.5 * r2);
+                eLead[i * ldr + r] = __dmul_rn(s2, exp(-0.5 * r2));
             }
         }
         __syncthreads();
@@ -251,9 +255,14 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
             const double svg = causal ? sqrt(vg) : 0.0;
             double ss;
             if constexpr (SEP) posterior_sep<NREG>(sm, n, eLast + jj, ldl, eLead + (int)(row - row_first), ldr, svg, mu, ss);
-            else posterior_at<NREG>(sm, n, d, x, svg, tid, mu, ss);
+            else {
+                double xl[CBO_MAX_D];
+#pragma unroll
+                for (int k = 0; k < CBO_MAX_D; ++k) xl[k] = x[k] * il;
+                posterior_at<NREG>(sm, n, d, xl, svg, s2, tid, mu, ss);
+            }
             mu += mg;
-            var = ((1.0 + vg) - ss) + 1e-10;
+            var = ((s2 + vg) - ss) + 1e-10;
             if (S.mu) S.mu[loc] = mu;
             if (S.var) S.var[loc] = var;
         }
@@ -335,6 +344,7 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
     const int n = S.n_int, d = S.d, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int r = lane >> 2, q = lane & 3;
     const bool causal = S.causal != 0;
+    const double s2 = S.hyper ? S.hyper[0] : 1.0, il = S.hyper ? 1.0 / S.hyper[1] : 1.0;
     const int p_last = S.points ? 1 : S.p[d - 1];
     const int nb = (n + 7) >> 3, ksn = (n + 3) >> 2;
 
@@ -370,14 +380,14 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
         al[i] = i < n ? S.alpha[i] : 0.0;
         sv[i] = (causal && i < n) ? S.sqrt_v_int[i] : 0.0;
     }
-    for (int i = tid; i < n * d; i += kMmaThreads) xs[i] = S.x_int[i];
+    for (int i = tid; i < n * d; i += kMmaThreads) xs[i] = S.x_int[i] * il;
     if (SEP) {
         const double* __restrict__ gl = S.grid[d - 1];
         for (int e = tid; e < n4 * p_last; e += kMmaThreads) {
             const int i = e / p_last, j = e - i * p_last;
             double v = 0.0;
             if (i < n) {
-                const double t = gl[j] - S.x_int[i * d + d - 1];
+                const double t = (gl[j] - S.x_int[i * d + d - 1]) * il;
                 v = exp(-0.5 * (t * t));
             }
             eLast[i * ldl + j] = v;
@@ -392,11 +402,11 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
                 double r2 = 0.0;
                 for (int k = d - 2; k >= 0; --k) {
                     const long long pk = S.p[k];
-                    const double t = S.grid[k][(int)(rr % pk)] - S.x_int[i * d + k];
+                    const double t = (S.grid[k][(int)(rr % pk)] - S.x_int[i * d + k]) * il;
                     r2 = fma(t, t, r2);
                     rr /= pk;
                 }
-                v = exp(-0.5 * r2);
+                v = __dmul_rn(s2, exp(-0.5 * r2));
             }
             eLead[i * ldr + rw] = v;
         }
@@ -461,7 +471,7 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
             } else {
                 double xg[CBO_MAX_D];
 #pragma unroll
-                for (int k = 0; k < CBO_MAX_D; ++k) xg[k] = __shfl_sync(0xffffffffu, x[k], src);
+                for (int k = 0; k < CBO_MAX_D; ++k) xg[k] = __shfl_sync(0xffffffffu, x[k], src) * il;
 #pragma unroll
                 for (int ks = 0; ks < kMmaKS; ++ks) {
                     a[ks] = 0.0;
@@ -472,7 +482,7 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
                         for (int k = 0; k < CBO_MAX_D; ++k) {
                             if (k < d) { const double t = xg[k] - xs[jc * d + k]; r2 = fma(t, t, r2); }
                         }
-                        const double kv = exp(-0.5 * r2) + sv[jc] * svg_g;
+                        const double kv = fma(sv[jc], svg_g, __dmul_rn(s2, exp(-0.5 * r2)));
                         a[ks] = j < n ? kv : 0.0;
                         mp = fma(a[ks], al[jc], mp);
                     }
@@ -512,7 +522,7 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
             if (q == g) { mu = mp; ss = sp; }
         }
         mu += mg;
-        const double var = ((1.0 + vg) - ss) + 1e-10;
+        const double var = ((s2 + vg) - ss) + 1e-10;
         if (live) {
             if (S.mu) S.mu[loc] = mu;
             if (S.var) S.var[loc] = var;

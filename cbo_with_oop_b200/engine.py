@@ -18,8 +18,22 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import AcqGradOut, RefineResult, SetBest, SetDesc, SweepResult
+from ._lib import AcqGradOut, HyperResult, RefineResult, SetBest, SetDesc, SweepResult
 from .partition import SetSize, partition
+
+HYPER_S2_BOUNDS = (1e-6, 1e6)
+
+
+def hyper_bounds(grid: Sequence[np.ndarray]) -> np.ndarray:
+    """(s2_lo, s2_hi, l_lo, l_hi) of the marginal-likelihood fit of one exploration set's GP (cbo_posterior_hyper_fit):
+    s2 in [1e-6, 1e6]; l from the smallest grid spacing of the set (a shorter lengthscale only fits noise between
+    candidates the sweep never evaluates: unbounded, the fit runs to white-noise spikes far below one spacing) to ten
+    times the largest box span (beyond that the kernel is flat over the box).  A set whose box has no extent keeps l = 1."""
+    spans = [float(np.max(t) - np.min(t)) for t in grid]
+    steps = [sp / (len(t) - 1) for sp, t in zip(spans, grid) if len(t) > 1 and sp > 0.0]
+    if not steps:
+        return np.array([HYPER_S2_BOUNDS[0], HYPER_S2_BOUNDS[1], 1.0, 1.0])
+    return np.array([HYPER_S2_BOUNDS[0], HYPER_S2_BOUNDS[1], min(steps), 10.0 * max(spans)])
 
 
 @dataclass
@@ -110,7 +124,9 @@ def _round_up(x: int, m: int) -> int:
 class SweepEngine:
     def __init__(self, problems: Sequence[SetProblem], device: str | torch.device = "cuda:0", rank: int = 0,
                  world_size: int = 1, keep: Sequence[str] = (), process_group=None, n_int_capacity: int = _lib.CBO_MAX_NINT,
-                 pinned_staging: bool = False):
+                 pinned_staging: bool = False, fit_hyperparameters: bool = False):
+        """fit_hyperparameters: fit each set's GP variance and lengthscale by marginal likelihood on the device (K8) before
+        every posterior fit, instead of the reference's fixed (1, 1) (opt-in; off, every path and output is unchanged)."""
         if not torch.cuda.is_available():
             raise RuntimeError("SweepEngine needs a CUDA device: the CUDA library is the product, there is no CPU path")
         self.lib = _lib.load()
@@ -127,6 +143,7 @@ class SweepEngine:
         self.timing = False
         self._launch0 = self.lib.cbo_launch_count()
         self.pinned_staging = pinned_staging
+        self.fit_hyper = bool(fit_hyperparameters)
         for k in self.keep:
             if k not in ("mu", "var", "ei", "acq"):
                 raise ValueError(f"unknown array {k!r}")
@@ -180,6 +197,8 @@ class SweepEngine:
             b["m_int"] = self._dev((self.ncap,), zero=True)
             b["v_int"] = self._dev((self.ncap,), zero=True)
             b["fit_info"] = self._dev((2,), dtype=torch.int32, zero=True)
+            if self.fit_hyper:
+                b["hyper"] = torch.ones((2,), dtype=torch.float64, device=self.device)
             for k in range(d):
                 b[f"grid{k}"] = self._dev((len(pr.grid[k]),))
             for name in self.keep:
@@ -254,6 +273,7 @@ class SweepEngine:
             D.sqrt_v_int, D.m_int, D.v_int, D.fit_info = ptr("sqrt_v_int"), ptr("m_int"), ptr("v_int"), ptr("fit_info")
             D.mu, D.var, D.ei, D.acq = ptr("mu"), ptr("var"), ptr("ei"), ptr("acq")
             D.m, D.v = ptr("m"), ptr("v")
+            D.hyper = ptr("hyper")
             if pr.computes_prior:
                 N, c, Smc = pr.x_obs_int.shape[0], pr.x_obs_cond.shape[1], pr.mc_cond.shape[0]
                 D.c, D.n_obs, D.n_obs_pad = c, N, _round_up(N, _lib.CBO_NPAD)
@@ -446,6 +466,58 @@ class SweepEngine:
         if n:
             _lib.check(self.lib.cbo_posterior_fit(h, dptr, n, self._stream()), "cbo_posterior_fit")
 
+    def fit_hyperparameters(self, local_ids=None, max_iter: int = 100, gtol: float = 1e-6):
+        """K8 (cbo_posterior_hyper_fit) for all active sets or a contiguous run of local ids: the variance and lengthscale of
+        each set's GP by marginal likelihood on its current interventional data and prior at x_int (needs prior_eval(1)),
+        within hyper_bounds(grid), written to the set's hyper buffer that the posterior fit, the sweep and the refinement
+        read.  This is where the reference's models[i].optimize() (CBO.py:173) takes effect."""
+        if not self.fit_hyper:
+            raise ValueError("the engine was built with fit_hyperparameters=False: its sets have no hyper-parameter buffers")
+        h, dptr, n = self._subset(local_ids)
+        if not n:
+            return
+        first = 0 if local_ids is None else list(local_ids)[0]
+        ids = self.active[first:first + n]
+        bounds = np.ascontiguousarray(np.concatenate([hyper_bounds(self.problems[g].grid) for g in ids]), np.float64)
+        if getattr(self, "_hyper_res", None) is None:
+            self._hyper_res = torch.zeros((max(len(self.active), 1) * C.sizeof(HyperResult),), dtype=torch.uint8, device=self.device)
+            self._hyper_ws = torch.empty((max(self.lib.cbo_posterior_hyper_workspace_bytes(self.h_sets, len(self.active)), 256),),
+                                         dtype=torch.uint8, device=self.device)
+        _lib.check(self.lib.cbo_posterior_hyper_fit(h, dptr, n, bounds.ctypes.data_as(C.POINTER(C.c_double)), int(max_iter),
+                                                    float(gtol), C.c_void_p(self._hyper_ws.data_ptr()), self._hyper_ws.numel(),
+                                                    C.c_void_p(self._hyper_res.data_ptr() + first * C.sizeof(HyperResult)),
+                                                    self._stream()), "cbo_posterior_hyper_fit")
+
+    def hyperparameters(self, g: int):
+        """(variance, lengthscale) of global set g's GP: what K8 last fitted, or the reference's (1.0, 1.0)."""
+        if not self.fit_hyper:
+            return 1.0, 1.0
+        h = self.buf[self.local_of[g]]["hyper"].cpu().numpy()
+        return float(h[0]), float(h[1])
+
+    def hyper_result(self, g: int) -> Optional[dict]:
+        """K8's cbo_hyper_result of global set g from its last fit (None before the first fit)."""
+        if getattr(self, "_hyper_res", None) is None:
+            return None
+        li = self.local_of[g]
+        raw = self._hyper_res[li * C.sizeof(HyperResult):(li + 1) * C.sizeof(HyperResult)].cpu().numpy().tobytes()
+        r = HyperResult.from_buffer_copy(raw)
+        out = {n: getattr(r, n) for n, _ in HyperResult._fields_}
+        out["status"] = _lib.HYPER_STATUS.get(r.status, str(r.status))
+        return out
+
+    def posterior_nll(self, g: int) -> np.ndarray:
+        """(-log p(y), d/dlog s2, d/dlog l) of global set g's GP at its current hyper-parameters (cbo_posterior_nll); needs
+        the set's prior at x_int on the device."""
+        h, dptr = self._local_desc(self.local_of[g])
+        out = torch.empty((3,), dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.cbo_posterior_nll(h, dptr, 1, C.c_void_p(out.data_ptr()), self._stream()), "cbo_posterior_nll")
+        return out.cpu().numpy()
+
+    def log_marginal_likelihood(self, g: int) -> float:
+        """log p(y) of global set g's GP (GPy's model.log_likelihood()), from cbo_posterior_nll."""
+        return -float(self.posterior_nll(g)[0])
+
     def _sweep_local(self, best: float, task: str):
         A = len(self.active)
         if task not in ("min", "max"):
@@ -509,6 +581,8 @@ class SweepEngine:
         self._timed("prior_eval_train", lambda: self.prior_eval(1), ev)
         self._prior_rows_valid = {g for g in self.active if self.problems[g].computes_prior}
         self._row_begin = {}
+        if self.fit_hyper:
+            self._timed("hyper_fit", self.fit_hyperparameters, ev)
         self._timed("posterior_fit", self.posterior_fit, ev)
         self._timed("prior_eval_grid", lambda: self.prior_eval(0), ev)
         self._timed("sweep", lambda: self._sweep_local(best, task), ev)
@@ -547,7 +621,7 @@ class SweepEngine:
         self._set_row_begin({g: self._row_begin.get(g, 0) for g in refit if g in self._prior_rows_valid})
         self._mark_cached(self._posterior_valid - set(refit))
         refit_local = [self.local_of[g] for g in refit if g in self.local_of]
-        if not self.timing and len(refit_local) <= 1 and self.active:
+        if not self.timing and not self.fit_hyper and len(refit_local) <= 1 and self.active:
             # the whole trial in one library call (cbo_refresh_trial): descriptor upload, the appended rows' table and prior,
             # the refit, the sweep and its reductions -- six launches, no Python between them
             li = refit_local[0] if refit_local else -1
@@ -574,6 +648,8 @@ class SweepEngine:
                 self._timed("prior_eval_train", lambda: self.prior_eval(1, li), ev)
                 self._prior_rows_valid.add(g)
                 self._row_begin.pop(g, None)
+            if self.fit_hyper:
+                self._timed("hyper_fit", lambda: self.fit_hyperparameters(li), ev)
             self._timed("posterior_fit", lambda: self.posterior_fit(li), ev)
         self._timed("sweep", lambda: self._sweep_local(best, task), ev)
         self._set_row_begin({})      # host flags back to neutral; the device copy follows with the next trial's upload

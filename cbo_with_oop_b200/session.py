@@ -17,8 +17,8 @@ from .engine import SetProblem, SweepEngine, SweepOutput
 
 
 class AcquisitionSession:
-    def __init__(self, problems: Sequence[SetProblem], device="cuda:0", keep: Sequence[str] = ()):
-        self.engine = SweepEngine(list(problems), device=device, keep=keep)
+    def __init__(self, problems: Sequence[SetProblem], device="cuda:0", keep: Sequence[str] = (), fit_hyperparameters: bool = False):
+        self.engine = SweepEngine(list(problems), device=device, keep=keep, fit_hyperparameters=fit_hyperparameters)
         self.num_sets = len(problems)
         self.prior_ready = False          # tables + prior precompute done
         self.grid_ready = False           # prior on the grid cached
@@ -35,6 +35,10 @@ class AcquisitionSession:
             self.engine.prior_precompute()
             self.prior_ready = True
 
+    def ensure_fit(self, g: int):
+        """Bring global set g's posterior (and, when fitted, its hyper-parameters) up to date with its data."""
+        self._ensure_fit(g)
+
     def _ensure_fit(self, g: int):
         self._ensure_prior()
         if g in self.stale_fit:
@@ -42,6 +46,8 @@ class AcquisitionSession:
             if self.engine.problems[g].computes_prior:
                 self.engine.build_tables(li)           # the interventional-row table follows x_int
                 self.engine.prior_eval(1, li)
+            if self.engine.fit_hyper:
+                self.engine.fit_hyperparameters(li)
             self.engine.posterior_fit(li)
             self.stale_fit.discard(g)
 

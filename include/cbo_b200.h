@@ -30,7 +30,7 @@ extern "C" {
 #define CBO_API
 #endif
 
-#define CBO_ABI_VERSION 8
+#define CBO_ABI_VERSION 9
 #define CBO_MAX_D 4          /* intervened dimensions per exploration set (reference uses 1..3) */
 #define CBO_MAX_C 8          /* conditioning dimensions of an observational GP */
 #define CBO_MAX_NINT 128     /* interventional rows per set (reference: 10 .. ~50) */
@@ -108,6 +108,10 @@ typedef struct cbo_set_desc {
                                   alpha_obs and kyinv from them (NULL: the caller supplies alpha_obs / kyinv itself) */
     const double* points;      /* NULL: tensor grid.  Otherwise (g_total, d) row-major candidates; then p[0] = g_total,
                                   p[1..] = 1, grid[] is unused and tab[0] is the (g_total, n_obs_pad) exp table of the points */
+    /* ---- hyper-parameters of the per-set GP (ABI 9) ------------------------------------------------ */
+    double* hyper;             /* NULL: the reference's RBF variance 1 and lengthscale 1.  Otherwise two device doubles
+                                  (s2, l) read by cbo_posterior_fit, cbo_sweep, cbo_acq_grad and cbo_refine, and written by
+                                  cbo_posterior_hyper_fit:  k(x, x') = s2 exp(-.5 |x - x'|^2 / l^2) [+ sqrt(v(x)) sqrt(v(x'))] */
 } cbo_set_desc;
 
 /* Result of one sweep on one rank. */
@@ -198,7 +202,8 @@ CBO_API long cbo_prior_pair_items(const cbo_set_desc* h_sets, int num_sets, int 
  * pair-table kernel: per work item, (live 8 x 8 blocks of the tile) x (pair + mean columns, padded to 16). */
 CBO_API double cbo_prior_eval_flops(const cbo_set_desc* h_sets, int num_sets, int num_sms);
 
-/* K2. one CTA per set: Gram of the interventional rows (CausalRBF.K, causal_kernels.py:45-62, or RBF),
+/* K2. one CTA per set: Gram of the interventional rows (CausalRBF.K, causal_kernels.py:45-62, or RBF; variance and
+ * lengthscale from `hyper`, 1 when it is NULL),
  * + (1e-10 + 1e-8) I, Cholesky with GPy's jitter-retry rule, alpha = Ky^-1 (y - m).
  * Replaces GPRegression(...) at GaussianProcessFactory.py:57-73 (GPy ExactGaussianInference). */
 CBO_API int cbo_posterior_fit(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, void* stream);
@@ -220,10 +225,45 @@ CBO_API int cbo_sweep(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, in
  * array (it carries the trial's n_int / int_row_begin / posterior_cached flags), evaluates the interventional-row table and
  * the prior of the rows [int_row_begin, n_int) of that set only, refits it, and sweeps every set -- sets marked
  * posterior_cached only refresh EI from their mu / var arrays (16 B per candidate).  refit_set = -1: sweep only.
- * Six launches and one 480 B x num_sets copy; the per-stage entry points above remain for callers that time the stages. */
+ * Six launches and one 488 B x num_sets copy; the per-stage entry points above remain for callers that time the stages. */
 CBO_API int cbo_refresh_trial(const cbo_set_desc* h_sets, cbo_set_desc* d_sets, int num_sets, int refit_set, double best,
                               int task_sign, void* d_workspace, size_t workspace_bytes, cbo_set_best* d_tile_best,
                               cbo_set_best* d_set_best, cbo_sweep_result* d_result, void* stream);
+
+/* K8. Marginal-likelihood fit of the per-set GP's hyper-parameters (opt-in).
+ * The reference calls models[i].optimize() after every intervention (CBO.py:173) and then rebuilds the model with l = 1,
+ * s2 = 1 (SURVEY.md App. B #16); this is the fit it meant to keep, of exactly the model cbo_posterior_fit then builds:
+ *   Ky = s2 exp(-.5 r^2 / l^2) [+ sqrt(v_int) sqrt(v_int)^T] + (1e-10 + 1e-8 + jitter) I ,  r = y - m_int (or y)
+ *   NLL = .5 r^T Ky^-1 r + sum log L_ii + .5 n log(2 pi)   (jitter: K2's rule, mean(diag) 1e-6 10^t, t = 0..4)
+ * cbo_posterior_nll: d_out[3 s .. 3 s + 2] = NLL and its derivatives in log s2 and log l at the set's current `hyper`
+ * (NULL = (1, 1)); one CTA per set, every set needs m_int / v_int (causal) and x_int / y_int on the device.
+ * cbo_posterior_hyper_fit: per set, CBO_HYPER_STARTS deterministic starts (start 0 = (1, 1) clipped to the box, the others
+ * a lattice from the bounds and var(r)), one CTA each, a projected BFGS in (log s2, log l) inside
+ * h_bounds[4 s .. 4 s + 3] = (s2_lo, s2_hi, l_lo, l_hi) (HOST memory: checked, then copied into the workspace) with Armijo backtracking (steps 1, 1/2, .., 1/128); stop when
+ * max |projected gradient| <= gtol or after max_iter line searches.  A reduction keeps each set's lowest NLL (ties: lowest
+ * start; NaN = +inf) and writes it through `hyper`; a set none of whose starts has a positive-definite Gram keeps its
+ * `hyper`.  Bit-identical across runs and independent of the other sets of the call.  Every set needs hyper != NULL. */
+#define CBO_HYPER_STARTS 9
+enum {
+    CBO_HYPER_CONVERGED = 0,          /* max |projected gradient| <= gtol */
+    CBO_HYPER_MAX_ITER = 1,           /* max_iter line searches done */
+    CBO_HYPER_LINE_SEARCH_FAILED = 2, /* no backtracking step lowered the NLL (Armijo) */
+    CBO_HYPER_NOT_PD = 3              /* the Gram was not positive definite, even with jitter, at every start: hyper unchanged */
+};
+typedef struct cbo_hyper_result {
+    double variance, lengthscale;  /* the set's (s2, l) after the call */
+    double nll;                    /* -log p(y) there */
+    double nll_start;              /* -log p(y) at (1, 1) (NaN if not positive definite there) */
+    int32_t iterations;            /* line searches of the winning start */
+    int32_t status;                /* CBO_HYPER_* of the winning start */
+    int32_t start;                 /* index of the winning start, -1 when none succeeded */
+    int32_t jitter_tries;          /* jitter retries of the Cholesky at the result */
+} cbo_hyper_result;
+CBO_API int cbo_posterior_nll(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, double* d_out, void* stream);
+CBO_API size_t cbo_posterior_hyper_workspace_bytes(const cbo_set_desc* h_sets, int num_sets);
+CBO_API int cbo_posterior_hyper_fit(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, const double* h_bounds,
+                                    int max_iter, double gtol, void* d_workspace, size_t workspace_bytes, cbo_hyper_result* d_out,
+                                    void* stream);
 
 /* K4 (multi-GPU). Combine `num_ranks` gathered per-set bests (rank-major: [rank][set]) into the global
  * per-set bests and the global result with the same rule on every rank.  Runs on the device so the

@@ -29,6 +29,10 @@ class ArgumentParser:
         self.parser.add_argument("--refine_acquisition", action="store_true",
                                  help="refine each exploration set's grid maximum off the grid with on-device gradients "
                                       "(the reference's L-BFGS polish); off: the grid argmax")
+        self.parser.add_argument("--optimize_surrogates", action="store_true",
+                                 help="fit each exploration set's GP variance and lengthscale by marginal likelihood on the "
+                                      "device at every refit (the reference's models[i].optimize(), whose result it discards); "
+                                      "off: the reference's fixed variance 1 and lengthscale 1")
 
     def parse(self, verbose=False, argv=None):
         args = self.parser.parse_args(argv)

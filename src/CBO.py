@@ -46,6 +46,8 @@ class CBO:
         self.observational_fit = getattr(args, "observational_fit", "device")
         # refine each set's grid maximum off the grid (SweepEngine.refine): the reference's continuous L-BFGS polish
         self.refine_acquisition = bool(getattr(args, "refine_acquisition", False))
+        # fit each set's GP variance / lengthscale by marginal likelihood at every refit (K8); off: the reference's (1, 1)
+        self.optimize_surrogates = bool(getattr(args, "optimize_surrogates", False))
 
         self.mean_functions, self.var_functions, self.models = [], [], []
         self.costs = self.graph.get_cost_structure(type_cost=self.type_cost)
@@ -154,7 +156,7 @@ class CBO:
                 problems.append(SetProblem.non_causal(self.monitor.space_list[s].grid_tables(self.grid_points_per_dim),
                                                       self.monitor.data_x[s], self.monitor.data_y[s].reshape(-1), fix, variable,
                                                       name="".join(variables)))
-            self._plain_session = AcquisitionSession(problems, device=self.device)
+            self._plain_session = AcquisitionSession(problems, device=self.device, fit_hyperparameters=self.optimize_surrogates)
         return self._plain_session
 
     def get_session(self):

@@ -103,5 +103,6 @@ class DoCalculus:
     def get_session(self):
         if self.session is None:
             from cbo_with_oop_b200.session import AcquisitionSession
-            self.session = AcquisitionSession([self.set_problem(s) for s in range(self.cbo.es_size)], device=self.cbo.device)
+            self.session = AcquisitionSession([self.set_problem(s) for s in range(self.cbo.es_size)], device=self.cbo.device,
+                                              fit_hyperparameters=getattr(self.cbo, "optimize_surrogates", False))
         return self.session

@@ -3,7 +3,11 @@
 The reference returns GPy GPRegression objects (optionally inside emukit's GPyModelWrapper); this build returns
 `SurrogateModel`, which has the surface the agent uses -- predict / set_data / optimize / X / Y -- and evaluates
 everything with the CUDA kernels: Gram + Cholesky + solves in csrc/posterior_fit.cu, predictive mean / variance / EI
-in csrc/sweep.cu.  Hyper-parameters are the reference's: lengthscale 1, variance 1, noise 1e-10 (:57-73)."""
+in csrc/sweep.cu.  Hyper-parameters are the reference's: lengthscale 1, variance 1, noise 1e-10 (:57-73), unless the agent
+runs with --optimize_surrogates: then the variance and lengthscale of every set are fitted by marginal likelihood on the
+device (csrc/posterior_hyper.cu) at each refit, and `kern` / `log_likelihood()` report them."""
+from types import SimpleNamespace
+
 from enum import IntEnum
 
 import numpy as np
@@ -139,8 +143,39 @@ class SurrogateModel:
     def optimize(self):
         """The reference re-optimises this GP's hyper-parameters after every intervention (CBO.py:173) and discards
         them when the model is rebuilt with lengthscale 1 / variance 1 before the next acquisition (CBO.py:229-235,
-        SURVEY.md Appendix B #16); keeping the fixed values is therefore behaviour-preserving."""
+        SURVEY.md Appendix B #16); keeping the fixed values is therefore behaviour-preserving.  With --optimize_surrogates
+        the fit the reference meant to keep moves to the refit itself: the session's next posterior fit of this set runs the
+        marginal-likelihood search first (SweepEngine.fit_hyperparameters), on the same data this call would have seen."""
         return None
+
+    @property
+    def hyperparameters(self):
+        """(variance, lengthscale) of the per-set GP as the kernels use them: the fitted values when the shared session
+        fits them (--optimize_surrogates), otherwise the reference's (1.0, 1.0)."""
+        shared = self._shared()
+        if shared is None:
+            return 1.0, 1.0
+        session, g = shared
+        session.mark_interventional(g, self.X, self.Y)
+        session.ensure_fit(g)
+        return session.engine.hyperparameters(g)
+
+    @property
+    def kern(self):
+        """GPy-shaped read access: model.kern.variance, model.kern.lengthscale."""
+        s2, l = self.hyperparameters
+        return SimpleNamespace(variance=s2, lengthscale=l)
+
+    def log_likelihood(self):
+        """log p(Y) of this GP at its current hyper-parameters (GPy's model.log_likelihood()), from cbo_posterior_nll."""
+        shared = self._shared()
+        if shared is not None:
+            session, g = shared
+            session.mark_interventional(g, self.X, self.Y)
+        else:
+            session, g = self._private_session([np.zeros(1)] * self.X.shape[1]), 0
+        session.ensure_fit(g)
+        return session.engine.log_marginal_likelihood(g)
 
     @property
     def model(self):          # emukit wrapper exposes the wrapped GPy model as .model
