@@ -1,13 +1,12 @@
 // K8 -- marginal-likelihood fit of the per-set GP's variance s2 and lengthscale l (opt-in), one CTA per (set, start), the
 // Gram resident in shared memory (n <= 128, as in K2).
 //
-// The model is exactly the one K2 then factors (csrc/posterior_fit.cu):
-//   Ky = s2 exp(-.5 r^2 / l^2) + sqrt(v) sqrt(v)^T [causal only] + (1e-10 + 1e-8 + jitter) I ,  res = y - m_int (or y)
+// The model, its Gram and jitchol are surrogate.cuh's, the same code K2 runs, so K8 optimises the model K2 then factors:
+//   Ky = s2 exp(-.5 r^2 / l^2) + sqrt(v) sqrt(v)^T [causal only] + (kSurrogateDiag + jitter) I ,  res = y - m_int (or y)
 //   NLL = .5 res^T alpha + sum log L_ii + .5 n log(2 pi) ,  alpha = Ky^-1 res
 //   dNLL / dtheta = .5 sum_ij (W - alpha alpha^T)_ij dK_ij / dtheta ,  W = Ky^-1 = L^-T L^-1 ,  theta = (log s2, log l)
 //   dK / dlog s2 = s2 E ,  dK / dlog l = s2 E o (r^2 / l^2) ,  E = exp(-.5 r^2 / l^2)
-// with K2's jitter rule (plain Cholesky, then mean(diag Ky) 1e-6 10^t, t = 0..4) and r^2 formed from coordinate differences
-// scaled by 1 / l.  The gradient needs L^-1 (n^3 / 6, written transposed into the strict upper triangle, which the Cholesky
+// The gradient needs L^-1 (n^3 / 6, written transposed into the strict upper triangle, which the Cholesky
 // leaves free) and one pass over the pairs i >= j for W_ij = sum_{k >= i} X_ki X_kj (another n^3 / 6): no second n x n array,
 // so n = 128 fits in 132 KB.  The row pitch is odd (n | 1): every access walks rows or columns without bank conflicts.
 //
@@ -20,7 +19,7 @@
 // state); reductions are fixed trees, so a result depends on its set and start alone: bit-identical across runs, across
 // calls that group the sets differently, and across ranks that run K8 redundantly on a split set.
 #include <float.h>
-#include "cbo_common.cuh"
+#include "surrogate.cuh"
 
 namespace cbo {
 
@@ -38,11 +37,11 @@ struct HypSmem {
     double* al;    // alpha
     double* dsq;   // L_ii
     double* rinv;  // 1 / L_ii
-    double* red;   // 2 kHypWarps reduction slots + scalars
+    double* red;   // 2 kHypWarps reduction slots, then the NLL
     int ld;
 };
 inline size_t hyp_smem_bytes(int n) {
-    return ((size_t)n * (n | 1) + (size_t)n * CBO_MAX_D + 5 * (size_t)n + 2 * kHypWarps + 4) * sizeof(double);
+    return ((size_t)n * (n | 1) + (size_t)n * CBO_MAX_D + 5 * (size_t)n + 2 * kHypWarps + 1) * sizeof(double);
 }
 
 __device__ void hyp_stage(const cbo_set_desc& S, HypSmem& sm, double* base) {
@@ -76,65 +75,22 @@ __device__ __forceinline__ void hyp_sum2(double& a, double& b, double* red) {
     for (int k = 0; k < kHypWarps; ++k) { a += red[2 * k]; b += red[2 * k + 1]; }
 }
 
-// NLL at (s2, l): Gram, Cholesky with K2's jitter rule, alpha.  Returns the jitter retries (0..5), or -1 when Ky is not
-// positive definite even with jitter (f = +inf).  Leaves L, dsq and alpha in shared memory for hyp_grad.
-__device__ int hyp_nll(const HypSmem& sm, int n, int d, double s2, double l, double& f) {
+// NLL at h: K2's Gram and jitchol (surrogate.cuh), then alpha.  Returns the jitter retries (0..5), or -1 when Ky is not
+// positive definite even with jitter (f = +inf).  Leaves L, dsq, rinv and alpha in shared memory for hyp_grad.
+__device__ int hyp_nll(const HypSmem& sm, int n, int d, SurrogateHyper h, double& f) {
     const int tid = threadIdx.x, ld = sm.ld;
-    const double il = 1.0 / l;
-    double* scal = sm.red + 2 * kHypWarps;     // [0] mean of diag Ky, [1] NLL
-    int tries = 0;
-    double jitter = 0.0;
-    for (;;) {
-        for (int e = tid; e < n * n; e += kHypThreads) {
-            const int i = e / n, j = e - i * n;
-            if (j > i) continue;
-            double r2 = 0.0;
-            for (int k = 0; k < d; ++k) {
-                const double t = (sm.xs[i * d + k] - sm.xs[j * d + k]) * il;
-                r2 = fma(t, t, r2);
-            }
-            double kij = fma(sm.sv[i], sm.sv[j], s2 * exp(-0.5 * r2));
-            if (i == j) kij += (1e-10 + 1e-8) + jitter;
-            sm.A[i * ld + j] = kij;
-        }
-        __syncthreads();
-        if (tries == 0) {
-            if (tid == 0) {
-                double t = 0.0;
-                for (int i = 0; i < n; ++i) t += sm.A[i * ld + i];
-                scal[0] = t / n;
-            }
-            __syncthreads();
-        }
-        // right-looking Cholesky, lower (K2's arithmetic; the pivot test is uniform over the CTA)
-        bool failed = false;
-        for (int j = 0; j < n; ++j) {
-            const double piv = sm.A[j * ld + j];
-            if (!(piv > 0.0)) { failed = true; break; }
-            const double sq = sqrt(piv);
-            const double inv = 1.0 / sq;
-            if (tid == 0) { sm.dsq[j] = sq; sm.rinv[j] = inv; }
-            for (int i = j + 1 + tid; i < n; i += kHypThreads) sm.A[i * ld + j] *= inv;
-            __syncthreads();
-            for (int i = j + 1 + (tid >> 4); i < n; i += kHypThreads / 16)
-                for (int k = j + 1 + (tid & 15); k <= i; k += 16) sm.A[i * ld + k] -= sm.A[i * ld + j] * sm.A[k * ld + j];
-            __syncthreads();
-        }
-        if (!failed) break;
-        __syncthreads();
-        if (tries == 5) { f = __longlong_as_double(0x7ff0000000000000LL); return -1; }
-        jitter = (tries == 0) ? scal[0] * 1e-6 : jitter * 10.0;
-        ++tries;
-    }
-    // z = L^-1 res, alpha = L^-T z in one warp (lane l owns rows l + 32 r); |z|^2 and sum log L_ii by fixed butterflies
+    double* nll = sm.red + 2 * kHypWarps;
+    const int tries = surrogate_jitchol<kHypThreads>(sm.A, ld, sm.xs, sm.sv, n, d, h, sm.dsq, sm.rinv);
+    if (tries < 0) { f = __longlong_as_double(0x7ff0000000000000LL); return -1; }
+    // z = L^-1 res, alpha = L^-T z in one warp as K2's warp_solve_lower / _upper, but multiplying by 1 / L_ii where K2
+    // divides by L_ii: the division lies on the dependent chain of every row, and with it the fit of a shipped configuration
+    // took up to 1.4x as long.  |z|^2 and sum log L_ii by fixed butterflies.
     if (tid < 32) {
         double z[4];
 #pragma unroll
         for (int r = 0; r < 4; ++r) z[r] = (tid + 32 * r < n) ? sm.res[tid + 32 * r] : 0.0;
         for (int j = 0; j < n; ++j) {
-            const int slot = j >> 5;
-            const double own = (slot == 0 ? z[0] : slot == 1 ? z[1] : slot == 2 ? z[2] : z[3]) * sm.rinv[j];
-            const double zj = __shfl_sync(0xffffffffu, own, j & 31);
+            const double zj = __shfl_sync(0xffffffffu, warp_own_row(z, j) * sm.rinv[j], j & 31);
 #pragma unroll
             for (int r = 0; r < 4; ++r) {
                 const int i = tid + 32 * r;
@@ -151,9 +107,7 @@ __device__ int hyp_nll(const HypSmem& sm, int n, int d, double s2, double l, dou
         zz = warp_sum(zz);
         lg = warp_sum(lg);
         for (int j = n - 1; j >= 0; --j) {
-            const int slot = j >> 5;
-            const double own = (slot == 0 ? z[0] : slot == 1 ? z[1] : slot == 2 ? z[2] : z[3]) * sm.rinv[j];
-            const double aj = __shfl_sync(0xffffffffu, own, j & 31);
+            const double aj = __shfl_sync(0xffffffffu, warp_own_row(z, j) * sm.rinv[j], j & 31);
 #pragma unroll
             for (int r = 0; r < 4; ++r) {
                 const int i = tid + 32 * r;
@@ -164,18 +118,18 @@ __device__ int hyp_nll(const HypSmem& sm, int n, int d, double s2, double l, dou
 #pragma unroll
         for (int r = 0; r < 4; ++r)
             if (tid + 32 * r < n) sm.al[tid + 32 * r] = z[r];
-        if (tid == 0) scal[1] = (0.5 * zz + lg) + n * kHalfLog2Pi;
+        if (tid == 0) *nll = (0.5 * zz + lg) + n * kHalfLog2Pi;
     }
     __syncthreads();
-    f = scal[1];
+    f = *nll;
     return tries;
 }
 
-// Gradient of the NLL in (log s2, log l) from the state hyp_nll left (same s2, l).
-__device__ void hyp_grad(const HypSmem& sm, int n, int d, double s2, double l, double& g0, double& g1) {
+// Gradient of the NLL in (log s2, log l) from the state hyp_nll left (same h).
+__device__ void hyp_grad(const HypSmem& sm, int n, int d, SurrogateHyper h, double& g0, double& g1) {
     const int tid = threadIdx.x, ld = sm.ld;
-    const double il = 1.0 / l;
-    // X = L^-1, column by column from the right: X_ij = -(sum_{j < k <= i} X_ik L_kj) / L_jj, stored at A[j][i]
+    // X = L^-1, column by column from the right: X_ij = -(sum_{j < k <= i} X_ik L_kj) / L_jj, stored at A[j][i].  (K2's
+    // surrogate_lower_inverse, which walks each column down its rows, made the fit 2-3.5 % slower here, 1.7 % at n = 128.)
     for (int j = n - 2; j >= 0; --j) {
         for (int i = j + 1 + tid; i < n; i += kHypThreads) {
             double a = sm.A[i * ld + j] * sm.rinv[i];
@@ -192,12 +146,8 @@ __device__ void hyp_grad(const HypSmem& sm, int n, int d, double s2, double l, d
         const double xij = (i == j) ? sm.rinv[i] : sm.A[j * ld + i];
         double w = xij * sm.rinv[i];
         for (int k = i + 1; k < n; ++k) w = fma(sm.A[i * ld + k], sm.A[j * ld + k], w);
-        double r2 = 0.0;
-        for (int k = 0; k < d; ++k) {
-            const double t = (sm.xs[i * d + k] - sm.xs[j * d + k]) * il;
-            r2 = fma(t, t, r2);
-        }
-        const double c = (i == j ? 0.5 : 1.0) * (w - sm.al[i] * sm.al[j]) * (s2 * exp(-0.5 * r2));
+        const double r2 = surrogate_r2(sm.xs, i, j, d, h.il);
+        const double c = (i == j ? 0.5 : 1.0) * (w - sm.al[i] * sm.al[j]) * surrogate_rbf(r2, h.s2);
         t0 += c;
         t1 = fma(c, r2, t1);
     }
@@ -239,22 +189,23 @@ hyper_fit_kernel(const cbo_set_desc* __restrict__ sets, const double* __restrict
         th[1] = lb[1] + (a + 0.5) * 0.25 * (ub[1] - lb[1]);
     }
     for (int k = 0; k < 2; ++k) th[k] = fmin(fmax(th[k], lb[k]), ub[k]);
+    auto at = [](const double (&t)[2]) { return SurrogateHyper{exp(t[0]), 1.0 / exp(t[1])}; };     // (log s2, log l) -> (s2, 1 / l)
     const double nan = __longlong_as_double(0x7ff8000000000000LL);
     double f, f11 = nan, g[2] = {0.0, 0.0};
-    int tries = hyp_nll(sm, n, d, exp(th[0]), exp(th[1]), f);
+    int tries = hyp_nll(sm, n, d, at(th), f);
     if (k0 == 0) {
         if (th[0] == 0.0 && th[1] == 0.0) f11 = tries >= 0 ? f : nan;
         else {
             double f1;
-            const int t1 = hyp_nll(sm, n, d, 1.0, 1.0, f1);
+            const int t1 = hyp_nll(sm, n, d, SurrogateHyper{1.0, 1.0}, f1);
             f11 = t1 >= 0 ? f1 : nan;
-            tries = hyp_nll(sm, n, d, exp(th[0]), exp(th[1]), f);     // L of the start point again, for its gradient
+            tries = hyp_nll(sm, n, d, at(th), f);     // L of the start point again, for its gradient
         }
     }
     int status = CBO_HYPER_MAX_ITER, iter = 0;
     if (tries < 0) status = CBO_HYPER_NOT_PD;
     else {
-        hyp_grad(sm, n, d, exp(th[0]), exp(th[1]), g[0], g[1]);
+        hyp_grad(sm, n, d, at(th), g[0], g[1]);
         if (!(isfinite(g[0]) && isfinite(g[1]))) status = CBO_HYPER_LINE_SEARCH_FAILED;
     }
     double H[4] = {1.0, 0.0, 0.0, 1.0};
@@ -286,7 +237,7 @@ hyper_fit_kernel(const cbo_set_desc* __restrict__ sets, const double* __restrict
         for (int j = 0; j < kHypTrials && !acc; ++j) {
             const double t = ldexp(1.0, -j);
             for (int k = 0; k < 2; ++k) tt[k] = fmin(fmax(fma(t, p[k], th[k]), lb[k]), ub[k]);
-            tr = hyp_nll(sm, n, d, exp(tt[0]), exp(tt[1]), ft);
+            tr = hyp_nll(sm, n, d, at(tt), ft);
             const double gain = fma(g[0], tt[0] - th[0], g[1] * (tt[1] - th[1]));
             acc = tr >= 0 && ft < f && ft <= fma(kHypArmijo, gain, f);     // NaN fails
         }
@@ -297,7 +248,7 @@ hyper_fit_kernel(const cbo_set_desc* __restrict__ sets, const double* __restrict
             break;
         }
         double gt[2];
-        hyp_grad(sm, n, d, exp(tt[0]), exp(tt[1]), gt[0], gt[1]);
+        hyp_grad(sm, n, d, at(tt), gt[0], gt[1]);
         if (!(isfinite(gt[0]) && isfinite(gt[1]))) { status = CBO_HYPER_LINE_SEARCH_FAILED; break; }
         const double sv[2] = {tt[0] - th[0], tt[1] - th[1]};
         const double yv[2] = {gt[0] - g[0], gt[1] - g[1]};
@@ -369,10 +320,10 @@ posterior_nll_kernel(const cbo_set_desc* __restrict__ sets, double* __restrict__
     HypSmem sm;
     hyp_stage(S, sm, smem_d);
     __syncthreads();
-    const double s2 = S.hyper ? S.hyper[0] : 1.0, l = S.hyper ? S.hyper[1] : 1.0;
+    const SurrogateHyper h = surrogate_hyper(S);
     double f, g0 = 0.0, g1 = 0.0;
-    const int tries = hyp_nll(sm, n, d, s2, l, f);
-    if (tries >= 0) hyp_grad(sm, n, d, s2, l, g0, g1);
+    const int tries = hyp_nll(sm, n, d, h, f);
+    if (tries >= 0) hyp_grad(sm, n, d, h, g0, g1);
     else f = g0 = g1 = __longlong_as_double(0x7ff8000000000000LL);
     if (threadIdx.x == 0) {
         out[3 * blockIdx.x] = f;

@@ -10,7 +10,7 @@
 //                   (each sum is accumulated with the weights a_kj themselves: no x_k u^T M u - sum_j X_kj ... cancellation)
 //   per-set GP      e_i = s2 exp(-.5 |x - x_i|^2 / l^2),  k*_i = e_i + sv_i sqrt(v) (non-causal: e_i, m = v = 0)
 //                   dk*_i = -e_i (x - x_i) / l^2 + sv_i dv / (2 sqrt v)     ((s2, l) = hyper, (1, 1) when NULL)
-//                   mu = m + k*.alpha,  var = (s2 + v) - |L^-1 k*|^2 + 1e-10   (as K3 computes them)
+//                   mu = m + k*.alpha,  var = (s2 + v) - |L^-1 k*|^2 + noise   (k*, var, EI and cost: surrogate.cuh)
 //                   dmu = dm + sum_i alpha_i dk*_i,  dvar = dv - 2 beta^T dk*,  beta = L^-T L^-1 k*
 //   acquisition     u = (best - mu) / sd,  ei = sign sd (u Phi + phi),  dei = -sign Phi dmu + sign phi dvar / (2 sd)
 //                   c = cost_fix + cost_variable sum |x_k|,  acq = ei / c,  dacq = (dei - acq dc) / c
@@ -32,6 +32,7 @@
 // the gradient scaled so that its largest move is one grid spacing.
 #include <float.h>
 #include "dmma_tile.cuh"
+#include "surrogate.cuh"
 
 namespace cbo {
 
@@ -250,8 +251,9 @@ __device__ void stage_posterior(const cbo_set_desc& S, RefSmem& sm, double* base
     sm.al = sm.Lp + (size_t)n * (n + 1) / 2;
     sm.sv = sm.al + n;
     sm.xs = sm.sv + n;
-    sm.s2 = S.hyper ? S.hyper[0] : 1.0;
-    sm.il = S.hyper ? 1.0 / S.hyper[1] : 1.0;
+    const SurrogateHyper h = surrogate_hyper(S);
+    sm.s2 = h.s2;
+    sm.il = h.il;
     for (int e = threadIdx.x; e < n * n; e += blockDim.x) {
         const int i = e / n, j = e % n;
         if (j <= i) sm.Lp[i * (i + 1) / 2 + j] = S.L[e];
@@ -314,8 +316,8 @@ __device__ void eval_point(const cbo_set_desc& S, const RefSmem& sm, const doubl
                 z[k] = k < d ? xl[k] - sm.xs[i * d + k] : 0.0;
                 r2 = fma(z[k], z[k], r2);
             }
-            const double e = __dmul_rn(sm.s2, exp(-0.5 * r2));
-            ks[r] = fma(sm.sv[i], sqv, e);
+            const double e = surrogate_rbf(r2, sm.s2);
+            ks[r] = surrogate_k(r2, sm.sv[i], sqv, sm.s2);
 #pragma unroll
             for (int k = 0; k < CBO_MAX_D; ++k) dks[r][k] = fma(-e, __dmul_rn(z[k], sm.il), sm.sv[i] * dv[k] * hv);
             mu_p = fma(ks[r], sm.al[i], mu_p);
@@ -348,7 +350,7 @@ __device__ void eval_point(const cbo_set_desc& S, const RefSmem& sm, const doubl
 #pragma unroll
     for (int r = 0; r < 4; ++r) ss = fma(rr[r], rr[r], ss);
     ss = warp_sum(ss);
-    const double var = ((sm.s2 + v) - ss) + 1e-10;
+    const double var = surrogate_var(sm.s2, v, ss);
     // beta = L^-T t (backward substitution; lane j % 32 owns beta_j)
 #pragma unroll
     for (int rb = 3; rb >= 0; --rb) {
@@ -373,24 +375,14 @@ __device__ void eval_point(const cbo_set_desc& S, const RefSmem& sm, const doubl
         for (int r = 0; r < 4; ++r) s = fma(rr[r], dks[r][k], s);
         dvar[k] = dv[k] - 2.0 * warp_sum(s);
     }
-    // EI and cost exactly as K3 evaluates them
-    const double sd = sqrt(var);
-    const double u = (best - mu) / sd;
-    const double pdf = 0.3989422804014326779 * exp(-0.5 * u * u);
-    const double cdf = 0.5 * erfc(-u * 0.7071067811865475244);
-    const double ei = task_sign * (sd * (u * cdf + pdf));
-    double cost = S.cost_fix;
-    if (S.cost_variable) {
-#pragma unroll
-        for (int k = 0; k < CBO_MAX_D; ++k)
-            if (k < d) cost += fabs(x[k]);
-    }
-    const double acq = ei / cost;
-    o.m = m; o.v = v; o.mu = mu; o.var = var; o.ei = ei; o.acq = acq;
+    const ExpectedImprovement e = expected_improvement(best, mu, var, task_sign);
+    const double cost = candidate_cost(S, d, x);
+    const double acq = e.ei / cost;
+    o.m = m; o.v = v; o.mu = mu; o.var = var; o.ei = e.ei; o.acq = acq;
 #pragma unroll
     for (int k = 0; k < CBO_MAX_D; ++k) {
         const double dc = (S.cost_variable && k < d) ? (x[k] > 0.0 ? 1.0 : (x[k] < 0.0 ? -1.0 : 0.0)) : 0.0;
-        const double dei = task_sign * (pdf * dvar[k] / (2.0 * sd) - cdf * dmu[k]);
+        const double dei = task_sign * (e.pdf * dvar[k] / (2.0 * e.sd) - e.cdf * dmu[k]);
         o.dm[k] = dm[k]; o.dv[k] = dv[k]; o.dmu[k] = dmu[k]; o.dvar[k] = dvar[k]; o.dei[k] = dei;
         o.dacq[k] = (dei - acq * dc) / cost;
     }

@@ -3,8 +3,8 @@
 // Per candidate x of set s (one thread each; L, alpha, X_I staged once per CTA in shared memory):
 //   k*_i = s2 exp(-.5 |x - X_I,i|^2 / l^2) + sqrt(v_I,i) sqrt(v(x))   CausalRBF.K(X_I, x), causal_kernels.py:55-62
 //   mu   = m(x) + k*.alpha                                           GPy PosteriorExact._raw_predict + mean function
-//   t    = L^-1 k* ; var = (s2 + v(x)) - |t|^2 + 1e-10               Kdiag :64-79, dtrtrs, Gaussian noise
-//   (s2, l) = cbo_set_desc.hyper, (1, 1) when NULL.  1 / l scales the staged coordinates (x_int, the candidate, the
+//   t    = L^-1 k* ; var = (s2 + v(x)) - |t|^2 + noise               Kdiag :64-79, dtrtrs, Gaussian noise
+//   (s2, l) = surrogate_hyper(S).  1 / l scales the staged coordinates (x_int, the candidate, the
 //   differences behind the separable tables) once, s2 is folded into the leading-dimension table and the A fragments: the
 //   per-candidate arithmetic is unchanged, and at (1, 1) every product is by 1.0, so the results are those of l = s2 = 1.
 //          (forward substitution for n <= 16 and n > 48; a DMMA product with L^-1 for 16 < n <= 48: sweep_mma_kernel)
@@ -14,10 +14,12 @@
 // tallied), per tile -> per set -> global (CBO.select_next_intervention, CBO.py:269-277: first set attaining the max).
 // The variance is not clipped (the reference does not clip either); a negative variance gives NaN.
 // Sets whose posterior is cached (cbo_set_desc.posterior_cached) only refresh EI from mu / var: ei_refresh_kernel.
+// k*, var, EI, the cost, the candidate's coordinates and the argmax reduction are surrogate.cuh's (shared with K2, K7, K8);
+// the separable k* tables below are a different factorisation of k* and keep their own form.
 // Roofline: with the prior cached this pass is 16 B/candidate of HBM reads plus n^2/2 FMAs; it is a few
 // per cent of a post-observation sweep and half of a post-intervention trial.
 #include <float.h>
-#include "cbo_common.cuh"
+#include "surrogate.cuh"
 
 namespace cbo {
 
@@ -50,7 +52,7 @@ __device__ __forceinline__ void posterior_at(const SweepSmem& sm, int n, int d, 
                 for (int k = 0; k < CBO_MAX_D; ++k) {
                     if (k < d) { const double q = x[k] - sm.xs[i * d + k]; r2 = fma(q, q, r2); }
                 }
-                const double ks = fma(sm.sv[i], svg, __dmul_rn(s2, exp(-0.5 * r2)));
+                const double ks = surrogate_k(r2, sm.sv[i], svg, s2);
                 mu = fma(ks, sm.al[i], mu);
                 const double* __restrict__ Li = sm.Lp + i * (i + 1) / 2;
                 // four interleaved partial sums: the row's dot product is a dependent FMA chain, and with 3-5 CTAs per SM
@@ -74,7 +76,7 @@ __device__ __forceinline__ void posterior_at(const SweepSmem& sm, int n, int d, 
             for (int k = 0; k < CBO_MAX_D; ++k) {
                 if (k < d) { const double q = x[k] - sm.xs[i * d + k]; r2 = fma(q, q, r2); }
             }
-            const double ks = fma(sm.sv[i], svg, __dmul_rn(s2, exp(-0.5 * r2)));
+            const double ks = surrogate_k(r2, sm.sv[i], svg, s2);
             mu = fma(ks, sm.al[i], mu);
             const double* __restrict__ Li = sm.Lp + i * (i + 1) / 2;
             double a = ks;
@@ -154,7 +156,7 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
     const int n = S.n_int, d = S.d, tid = threadIdx.x;
     const bool causal = S.causal != 0;
     const bool cached = S.posterior_cached != 0;   // mu / var of an earlier sweep are still valid: EI refresh only
-    const double s2 = S.hyper ? S.hyper[0] : 1.0, il = S.hyper ? 1.0 / S.hyper[1] : 1.0;
+    const auto [s2, il] = surrogate_hyper(S);
     if (sweep_class(S) != (NREG == 0 ? kClsGeneric : (SEP ? kClsFmaSep : kClsFma))) return;       // another launch's set
     const bool sep = SEP;
     const int p_last = S.points ? 1 : S.p[d - 1];
@@ -168,9 +170,6 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
     const int ldl = p_last | 1, ldr = sweep_lead_rows(S) | 1;          // odd pitches: no bank conflicts
     double* eLast = sm.tcol;                       // [n][ldl]
     double* eLead = eLast + (size_t)n * ldl;       // [n][ldr]
-    __shared__ double red_v[kSweepThreads / 32];
-    __shared__ long long red_i[kSweepThreads / 32];
-    __shared__ int red_n[kSweepThreads / 32];
 
     const long long loc0 = (long long)tile * CBO_SWEEP_TILE;
     const long long left = S.g_count - loc0;
@@ -231,20 +230,7 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
         double x[CBO_MAX_D];
 #pragma unroll
         for (int k = 0; k < CBO_MAX_D; ++k) x[k] = 0.0;
-        if (need_x) {
-            if (S.points) {  // explicit candidates
-#pragma unroll
-                for (int k = 0; k < CBO_MAX_D; ++k) x[k] = k < d ? S.points[gidx * d + k] : 0.0;
-            } else {
-                long long rr = row;
-                x[d - 1] = S.grid[d - 1][jj];
-                for (int k = d - 2; k >= 0; --k) {
-                    const long long pk = S.p[k];
-                    x[k] = S.grid[k][(int)(rr % pk)];
-                    rr /= pk;
-                }
-            }
-        }
+        if (need_x) candidate_x(S, d, gidx, row, jj, x);
         double mu, var;
         if (cached) {
             mu = S.mu[loc];
@@ -262,22 +248,12 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
                 posterior_at<NREG>(sm, n, d, xl, svg, s2, tid, mu, ss);
             }
             mu += mg;
-            var = ((s2 + vg) - ss) + 1e-10;
+            var = surrogate_var(s2, vg, ss);
             if (S.mu) S.mu[loc] = mu;
             if (S.var) S.var[loc] = var;
         }
-        const double sd = sqrt(var);
-        const double u = (best - mu) / sd;
-        const double pdf = 0.3989422804014326779 * exp(-0.5 * u * u);
-        const double cdf = 0.5 * erfc(-u * 0.7071067811865475244);
-        const double ei = task_sign * (sd * (u * cdf + pdf));
-        double cost = S.cost_fix;
-        if (S.cost_variable) {
-#pragma unroll
-            for (int k = 0; k < CBO_MAX_D; ++k)
-                if (k < d) cost += fabs(x[k]);
-        }
-        const double acq = ei / cost;
+        const double ei = expected_improvement(best, mu, var, task_sign).ei;
+        const double acq = ei / candidate_cost(S, d, x);
         if (S.ei) S.ei[loc] = ei;
         if (S.acq) S.acq[loc] = acq;
         if (acq != acq) ++n_nan;
@@ -286,23 +262,10 @@ sweep_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, d
         while (jj >= p_last && !S.points) { jj -= p_last; ++row; }
     }
     // first-argmax over the tile
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double ov = __shfl_xor_sync(0xffffffffu, val, o);
-        const long long oi = __shfl_xor_sync(0xffffffffu, idx, o);
-        n_nan += __shfl_xor_sync(0xffffffffu, n_nan, o);
-        if (better(ov, oi, val, idx)) { val = ov; idx = oi; }
-    }
-    if ((tid & 31) == 0) { red_v[tid >> 5] = val; red_i[tid >> 5] = idx; red_n[tid >> 5] = n_nan; }
-    __syncthreads();
+    cta_first_argmax<kSweepThreads>(val, idx, n_nan);
     if (tid == 0) {
-        int nan_total = red_n[0];
-        for (int x = 1; x < kSweepThreads / 32; ++x) {
-            if (better(red_v[x], red_i[x], val, idx)) { val = red_v[x]; idx = red_i[x]; }
-            nan_total += red_n[x];
-        }
         cbo_set_best b;
-        b.value = val; b.index = idx; b.n_nan = nan_total; b.reserved = 0;
+        b.value = val; b.index = idx; b.n_nan = n_nan; b.reserved = 0;
         tile_best[blockIdx.x] = b;
     }
 }
@@ -344,7 +307,7 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
     const int n = S.n_int, d = S.d, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int r = lane >> 2, q = lane & 3;
     const bool causal = S.causal != 0;
-    const double s2 = S.hyper ? S.hyper[0] : 1.0, il = S.hyper ? 1.0 / S.hyper[1] : 1.0;
+    const auto [s2, il] = surrogate_hyper(S);
     const int p_last = S.points ? 1 : S.p[d - 1];
     const int nb = (n + 7) >> 3, ksn = (n + 3) >> 2;
 
@@ -356,9 +319,6 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
     const int ldl = sweep_mma_ldl(p_last), ldr = sweep_mma_lead_rows(p_last, chunk) | 1;
     const int n4 = 4 * ksn;                                     // table rows: n rounded up to whole k4 steps, the extra rows zero
     double* eLead = eLast + (size_t)n4 * ldl;                   // [n4][ldr]
-    __shared__ double red_v[kMmaThreads / 32];
-    __shared__ long long red_i[kMmaThreads / 32];
-    __shared__ int red_n[kMmaThreads / 32];
 
     const long long loc0 = (long long)tile * CBO_SWEEP_TILE;
     const long long left = S.g_count - loc0;
@@ -435,20 +395,7 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
             lrow = (int)(off / (unsigned)p_last);
             jj = (int)(off - (unsigned)lrow * (unsigned)p_last);
         }
-        if (!SEP || S.cost_variable) {
-            if (S.points) {
-#pragma unroll
-                for (int k = 0; k < CBO_MAX_D; ++k) x[k] = k < d ? S.points[gidx * d + k] : 0.0;
-            } else {
-                long long rr = row_first + lrow;
-                x[d - 1] = S.grid[d - 1][jj];
-                for (int k = d - 2; k >= 0; --k) {
-                    const long long pk = S.p[k];
-                    x[k] = S.grid[k][(int)(rr % pk)];
-                    rr /= pk;
-                }
-            }
-        }
+        if (!SEP || S.cost_variable) candidate_x(S, d, gidx, row_first + lrow, jj, x);
         double mu = 0.0, ss = 0.0;
 #pragma unroll 1
         for (int g = 0; g < 4; ++g) {
@@ -482,7 +429,7 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
                         for (int k = 0; k < CBO_MAX_D; ++k) {
                             if (k < d) { const double t = xg[k] - xs[jc * d + k]; r2 = fma(t, t, r2); }
                         }
-                        const double kv = fma(sv[jc], svg_g, __dmul_rn(s2, exp(-0.5 * r2)));
+                        const double kv = surrogate_k(r2, sv[jc], svg_g, s2);
                         a[ks] = j < n ? kv : 0.0;
                         mp = fma(a[ks], al[jc], mp);
                     }
@@ -522,23 +469,13 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
             if (q == g) { mu = mp; ss = sp; }
         }
         mu += mg;
-        const double var = ((s2 + vg) - ss) + 1e-10;
+        const double var = surrogate_var(s2, vg, ss);
         if (live) {
             if (S.mu) S.mu[loc] = mu;
             if (S.var) S.var[loc] = var;
         }
-        const double sd = sqrt(var);
-        const double u = (best - mu) / sd;
-        const double pdf = 0.3989422804014326779 * exp(-0.5 * u * u);
-        const double cdf = 0.5 * erfc(-u * 0.7071067811865475244);
-        const double ei = task_sign * (sd * (u * cdf + pdf));
-        double cost = S.cost_fix;
-        if (S.cost_variable) {
-#pragma unroll
-            for (int k = 0; k < CBO_MAX_D; ++k)
-                if (k < d) cost += fabs(x[k]);
-        }
-        const double acq = ei / cost;
+        const double ei = expected_improvement(best, mu, var, task_sign).ei;
+        const double acq = ei / candidate_cost(S, d, x);
         if (live) {
             if (S.ei) S.ei[loc] = ei;
             if (S.acq) S.acq[loc] = acq;
@@ -547,23 +484,10 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
         }
     }
     // first-argmax over the tile
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double ov = __shfl_xor_sync(0xffffffffu, val, o);
-        const long long oi = __shfl_xor_sync(0xffffffffu, idx, o);
-        n_nan += __shfl_xor_sync(0xffffffffu, n_nan, o);
-        if (better(ov, oi, val, idx)) { val = ov; idx = oi; }
-    }
-    if (lane == 0) { red_v[warp] = val; red_i[warp] = idx; red_n[warp] = n_nan; }
-    __syncthreads();
+    cta_first_argmax<kMmaThreads>(val, idx, n_nan);
     if (tid == 0) {
-        int nan_total = red_n[0];
-        for (int w = 1; w < kMmaThreads / 32; ++w) {
-            if (better(red_v[w], red_i[w], val, idx)) { val = red_v[w]; idx = red_i[w]; }
-            nan_total += red_n[w];
-        }
         cbo_set_best b;
-        b.value = val; b.index = idx; b.n_nan = nan_total; b.reserved = 0;
+        b.value = val; b.index = idx; b.n_nan = n_nan; b.reserved = 0;
         tile_best[blockIdx.x] = b;
     }
     const int items_here = (cnt + CBO_SWEEP_TILE - 1) / CBO_SWEEP_TILE;
@@ -578,7 +502,7 @@ sweep_mma_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double bes
 // After an intervention every set but the refitted one keeps mu / var (cbo_set_desc.posterior_cached) and only EI moves with
 // the incumbent: 16 B per candidate and ~150 FP64 operations (sqrt, two divisions, exp, erfc).  Inside sweep_kernel's
 // one-candidate-at-a-time loop that chain was latency-bound (32 us per 1e6 candidates, 0.5 TB/s); here a thread carries
-// kEiUnroll independent candidates through it.  Same expressions in the same order as sweep_kernel: bit-identical results.
+// kEiUnroll independent candidates through it.  EI is surrogate.cuh's expected_improvement(), as in sweep_kernel: the same bits.
 constexpr int kEiUnroll = 4;
 __global__ void __launch_bounds__(kSweepThreads, 6)
 ei_refresh_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double best, double task_sign,
@@ -588,9 +512,6 @@ ei_refresh_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double be
     const cbo_set_desc& S = sets[s];
     if (sweep_class(S) != kClsCached) return;
     const int tid = threadIdx.x;
-    __shared__ double red_v[kSweepThreads / 32];
-    __shared__ long long red_i[kSweepThreads / 32];
-    __shared__ int red_n[kSweepThreads / 32];
     const long long loc0 = (long long)tile * CBO_SWEEP_TILE;
     const long long left = S.g_count - loc0;
     const int cnt = left < CBO_SWEEP_TILE ? (int)left : CBO_SWEEP_TILE;
@@ -614,11 +535,7 @@ ei_refresh_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double be
         }
 #pragma unroll
         for (int u = 0; u < kEiUnroll; ++u) {
-            const double sd = sqrt(var[u]);
-            const double z = (best - mu[u]) / sd;
-            const double pdf = 0.3989422804014326779 * exp(-0.5 * z * z);
-            const double cdf = 0.5 * erfc(-z * 0.7071067811865475244);
-            ei[u] = task_sign * (sd * (z * cdf + pdf));
+            ei[u] = expected_improvement(best, mu[u], var[u], task_sign).ei;
             acq[u] = ei[u] / cost;
         }
 #pragma unroll
@@ -632,23 +549,10 @@ ei_refresh_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double be
             }
         }
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double ov = __shfl_xor_sync(0xffffffffu, val, o);
-        const long long oi = __shfl_xor_sync(0xffffffffu, idx, o);
-        n_nan += __shfl_xor_sync(0xffffffffu, n_nan, o);
-        if (better(ov, oi, val, idx)) { val = ov; idx = oi; }
-    }
-    if ((tid & 31) == 0) { red_v[tid >> 5] = val; red_i[tid >> 5] = idx; red_n[tid >> 5] = n_nan; }
-    __syncthreads();
+    cta_first_argmax<kSweepThreads>(val, idx, n_nan);
     if (tid == 0) {
-        int nan_total = red_n[0];
-        for (int w = 1; w < kSweepThreads / 32; ++w) {
-            if (better(red_v[w], red_i[w], val, idx)) { val = red_v[w]; idx = red_i[w]; }
-            nan_total += red_n[w];
-        }
         cbo_set_best b;
-        b.value = val; b.index = idx; b.n_nan = nan_total; b.reserved = 0;
+        b.value = val; b.index = idx; b.n_nan = n_nan; b.reserved = 0;
         tile_best[blockIdx.x] = b;
     }
 }
@@ -657,9 +561,6 @@ ei_refresh_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, double be
 __global__ void __launch_bounds__(256)
 set_reduce_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, const cbo_set_best* __restrict__ tile_best,
                   cbo_set_best* __restrict__ set_best) {
-    __shared__ double rv[8];
-    __shared__ long long ri[8];
-    __shared__ int rn[8];
     const int s = blockIdx.x, tid = threadIdx.x;
     long long base = 0;
     for (int x = 0; x < s; ++x) base += host_items(sets[x], kItemsSweep);
@@ -672,21 +573,8 @@ set_reduce_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, const cbo
         if (better(b.value, b.index, val, idx)) { val = b.value; idx = b.index; }
         nn += b.n_nan;
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double ov = __shfl_xor_sync(0xffffffffu, val, o);
-        const long long oi = __shfl_xor_sync(0xffffffffu, idx, o);
-        nn += __shfl_xor_sync(0xffffffffu, nn, o);
-        if (better(ov, oi, val, idx)) { val = ov; idx = oi; }
-    }
-    if ((tid & 31) == 0) { rv[tid >> 5] = val; ri[tid >> 5] = idx; rn[tid >> 5] = nn; }
-    __syncthreads();
+    cta_first_argmax<256>(val, idx, nn);
     if (tid == 0) {
-        nn = rn[0];
-        for (int x = 1; x < 8; ++x) {
-            if (better(rv[x], ri[x], val, idx)) { val = rv[x]; idx = ri[x]; }
-            nn += rn[x];
-        }
         cbo_set_best b;
         b.value = val; b.index = (idx == LLONG_MAX) ? -1 : idx; b.n_nan = nn; b.reserved = 0;
         set_best[s] = b;
