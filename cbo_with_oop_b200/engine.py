@@ -19,7 +19,8 @@ import torch
 
 from . import _lib
 from ._lib import AcqGradOut, HyperResult, RefineResult, SetBest, SetDesc, SweepResult
-from .partition import SetSize, partition
+from .dist import gather_set_bests
+from .partition import SetSize, partition, refine_owners
 
 HYPER_S2_BOUNDS = (1e-6, 1e6)
 
@@ -121,6 +122,41 @@ def _round_up(x: int, m: int) -> int:
     return (x + m - 1) // m * m
 
 
+def grid_point(pr: SetProblem, index: int) -> np.ndarray:
+    """(d,) coordinates of flat grid index `index` of a set."""
+    ii = np.unravel_index(int(index), [len(t) for t in pr.grid])
+    return np.array([pr.grid[k][ii[k]] for k in range(pr.d)])
+
+
+def refined_output(out: SweepOutput, problems: Sequence[SetProblem], owners: Sequence[int], gathered: bytes) -> SweepOutput:
+    """Host assembly of SweepEngine.refine from the all-gathered cbo_refine_result tables (rank-major, one row of S records
+    per rank): set g's record is the one in the row of owners[g] (partition.refine_owners; -1: no record, the set keeps its
+    grid result).  A set whose record strictly improved on its start takes the refined value and coordinates; the selection
+    is the sweep's rule (first maximum, NaN = -inf)."""
+    S = len(problems)
+    rows = (RefineResult * (len(gathered) // C.sizeof(RefineResult))).from_buffer_copy(gathered)
+    grid_x = [grid_point(problems[g], out.set_indices[g]) if out.set_indices[g] >= 0 else None for g in range(S)]
+    values = np.array(out.set_values, np.float64, copy=True)
+    set_x = list(grid_x)
+    status = ["skipped_nonfinite"] * S
+    for g in range(S):
+        if owners[g] < 0:
+            continue
+        r = rows[owners[g] * S + g]
+        status[g] = _lib.REFINE_STATUS.get(r.status, str(r.status))
+        if r.value > r.start_value:          # strictly improved (both finite)
+            values[g] = r.value
+            set_x[g] = np.array(r.x[:problems[g].d])
+    valid = np.flatnonzero(np.asarray(out.set_indices) >= 0)
+    s, value, x = -1, out.value, None
+    if valid.size:
+        v = np.where(np.isnan(values[valid]), -np.inf, values[valid])
+        s = int(valid[int(np.argmax(v))])
+        value, x = float(values[s]), set_x[s]
+    return SweepOutput(s, int(out.set_indices[s]) if s >= 0 else out.index, value, x, values,
+                       np.array(out.set_indices, copy=True), out.n_nan, dict(out.stage_ms), set_x=set_x, refine_status=status)
+
+
 class SweepEngine:
     def __init__(self, problems: Sequence[SetProblem], device: str | torch.device = "cuda:0", rank: int = 0,
                  world_size: int = 1, keep: Sequence[str] = (), process_group=None, n_int_capacity: int = _lib.CBO_MAX_NINT,
@@ -149,7 +185,9 @@ class SweepEngine:
                 raise ValueError(f"unknown array {k!r}")
         S = len(self.problems)
         sizes = [SetSize(p.g_total, p.x_obs_int.shape[0] if p.computes_prior else 0, p.x_int.shape[0]) for p in self.problems]
-        self.slices = partition(sizes, world_size)[rank]
+        slices = partition(sizes, world_size)
+        self.slices = slices[rank]
+        self.refine_owner = refine_owners(slices)                       # global id -> the rank that refines the set
         self.active = [s for s in range(S) if self.slices[s][1] > 0]   # global ids of the sets this rank touches
         self.local_of = {g: i for i, g in enumerate(self.active)}
         self._alloc()
@@ -529,6 +567,17 @@ class SweepEngine:
                                           C.c_void_p(self.local_best.data_ptr()), C.c_void_p(self.result.data_ptr()),
                                           self._stream()), "cbo_sweep")
 
+    def _to_global(self, local: torch.Tensor, table: torch.Tensor, rec: int):
+        """Scatter this rank's records of its active sets (local ids, `rec` bytes each) into a global-indexed table."""
+        if self.active:
+            if not hasattr(self, "_active_idx"):
+                self._active_idx = torch.as_tensor(self.active, device=self.device, dtype=torch.long)
+            table.view(-1, rec).index_copy_(0, self._active_idx, local.view(-1, rec)[:len(self.active)])
+
+    def _all_gather(self, table: torch.Tensor, gathered: torch.Tensor):
+        """All-gather of a global-indexed per-set table over the engine's ranks, rank-major (NCCL; one rank: a copy)."""
+        gather_set_bests(table, gathered, self.world, self.group)
+
     def _finish(self, events) -> SweepOutput:
         """Scatter the local per-set bests into the global table, all-gather over ranks (NCCL), combine on
         the device with the same deterministic rule on every rank, and read the 24-byte result back."""
@@ -536,19 +585,10 @@ class SweepEngine:
         gb = self.global_best
         if not self._direct:
             gb.copy_(self._empty_best)
-            gv, lv = gb.view(S, sb), self.local_best.view(-1, sb)
-            if self.active:
-                if not hasattr(self, "_active_idx"):
-                    self._active_idx = torch.as_tensor(self.active, device=self.device, dtype=torch.long)
-                gv.index_copy_(0, self._active_idx, lv[:len(self.active)])
-            if self.world > 1:
-                from .dist import gather_set_bests
-                gather_set_bests(gb, self.gathered, self.world, self.group)
-                src, nr = self.gathered, self.world
-            else:   # combine_kernel's input and output must not alias (both are __restrict__): stage the table like a 1-rank gather
-                self.gathered[:gb.numel()].copy_(gb)
-                src, nr = self.gathered, 1
-            _lib.check(self.lib.cbo_argmax_combine(C.c_void_p(src.data_ptr()), nr, S, C.c_void_p(gb.data_ptr()),
+            self._to_global(self.local_best, gb, sb)
+            # combine_kernel's input and output must not alias (both are __restrict__): one rank stages its table by a copy
+            self._all_gather(gb, self.gathered)
+            _lib.check(self.lib.cbo_argmax_combine(C.c_void_p(self.gathered.data_ptr()), self.world, S, C.c_void_p(gb.data_ptr()),
                                                    C.c_void_p(self.result.data_ptr()), self._stream()), "cbo_argmax_combine")
         # ONE device -> host read of the step's result, into pinned memory; wait on its event only
         self.out_host.copy_(self.out_buf, non_blocking=True)
@@ -767,55 +807,49 @@ class SweepEngine:
         (causal_optimizer.py:52-62).  Returns a copy of `out` whose set_values, set_x and refine_status are per set and whose
         set / value / x are chosen by the sweep's rule (first maximum, NaN = -inf); `index` stays the grid index the chosen
         set started from.  A set that is skipped (external prior, explicit points, no finite grid maximum) or that no step
-        improved keeps its grid index, value and coordinates bit for bit."""
-        if self.world > 1:
-            raise ValueError("refine runs on one GPU: a multi-GPU engine would need the refined per-set results all-gathered")
+        improved keeps its grid index, value and coordinates bit for bit.
+
+        On a multi-GPU engine this is a collective call, like sweep(), and `out` is the sweep's output (global indices):
+        each set is refined by one rank that holds it (partition.refine_owners), the refined records are all-gathered
+        (56 B per set and rank, stage_ms "refine_gather"), and every rank returns the same output, the one a single-GPU
+        engine returns."""
+        ev: list = []
+        table = self._refine_local(out, best, task, max_iter, gtol, ev)
+        gathered = torch.empty((self.world * table.numel(),), dtype=torch.uint8, device=self.device)
+        self._timed("refine_gather", lambda: self._all_gather(table, gathered), ev)
+        return self._refine_finish(out, gathered, ev)
+
+    def _refine_local(self, out: SweepOutput, best: float, task: str, max_iter: int, gtol: float, ev: list) -> torch.Tensor:
+        """This rank's share of refine(): one cbo_refine call over its active sets, in which each set the rank owns starts
+        at its grid argmax in `out` and every other set at a NaN row (K7 skips it).  Returns the records scattered into a
+        global-indexed device table of S cbo_refine_result (zeros where the rank has no record)."""
         if task not in ("min", "max"):
             raise ValueError("task must be 'min' or 'max'")
-        S, A = len(self.problems), len(self.active)
-        grid_x = [None] * S
-        for g in range(S):
-            if out.set_indices[g] >= 0:
-                pr = self.problems[g]
-                ii = np.unravel_index(int(out.set_indices[g]), [len(t) for t in pr.grid])
-                grid_x[g] = np.array([pr.grid[k][ii[k]] for k in range(pr.d)])
+        S, A, rb = len(self.problems), len(self.active), C.sizeof(RefineResult)
         x0 = np.full((max(A, 1), _lib.CBO_MAX_D), np.nan)
         for li, g in enumerate(self.active):
-            if grid_x[g] is not None and np.isfinite(out.set_values[g]):
-                x0[li, :self.problems[g].d] = grid_x[g]
-        ev: list = []
-        res = None
+            if self.refine_owner[g] == self.rank and out.set_indices[g] >= 0 and np.isfinite(out.set_values[g]):
+                x0[li, :self.problems[g].d] = grid_point(self.problems[g], out.set_indices[g])
+        table = torch.zeros((S * rb,), dtype=torch.uint8, device=self.device)
         if A:
             self._push_descs()
             ws = self._refine_workspace(self.lib.cbo_refine_workspace_bytes(self.h_sets, A))
             d_x0 = torch.from_numpy(x0.reshape(-1)).to(self.device)
-            d_res = torch.empty((A * C.sizeof(RefineResult),), dtype=torch.uint8, device=self.device)
+            d_res = torch.empty((A * rb,), dtype=torch.uint8, device=self.device)
             self._timed("refine", lambda: _lib.check(self.lib.cbo_refine(
                 self.h_sets, C.c_void_p(self.d_sets.data_ptr()), A, float(best), 1 if task == "min" else -1,
                 C.c_void_p(d_x0.data_ptr()), int(max_iter), float(gtol), C.c_void_p(ws.data_ptr()), ws.numel(),
                 C.c_void_p(d_res.data_ptr()), self._stream()), "cbo_refine"), ev)
-            res = (RefineResult * A).from_buffer_copy(d_res.cpu().numpy().tobytes())
-        values = np.array(out.set_values, np.float64, copy=True)
-        set_x = list(grid_x)
-        status = ["skipped_nonfinite"] * S
-        for li, g in enumerate(self.active):
-            r = res[li]
-            status[g] = _lib.REFINE_STATUS.get(r.status, str(r.status))
-            if r.value > r.start_value:          # strictly improved (both finite)
-                values[g] = r.value
-                set_x[g] = np.array(r.x[:self.problems[g].d])
-        valid = np.flatnonzero(np.asarray(out.set_indices) >= 0)
-        s, value, x = -1, out.value, None
-        if valid.size:
-            v = np.where(np.isnan(values[valid]), -np.inf, values[valid])
-            s = int(valid[int(np.argmax(v))])
-            value, x = float(values[s]), set_x[s]
-        ms = dict(out.stage_ms)
+            self._to_global(d_res, table, rb)
+        return table
+
+    def _refine_finish(self, out: SweepOutput, gathered: torch.Tensor, ev: list) -> SweepOutput:
+        """Read the all-gathered tables back once and assemble the output (refined_output), the same on every rank."""
+        res = refined_output(out, self.problems, self.refine_owner, gathered.cpu().numpy().tobytes())
         for name, e0, e1 in ev:
             e1.synchronize()
-            ms[name] = ms.get(name, 0.0) + e0.elapsed_time(e1)
-        return SweepOutput(s, int(out.set_indices[s]) if s >= 0 else out.index, value, x, values,
-                           np.array(out.set_indices, copy=True), out.n_nan, ms, set_x=set_x, refine_status=status)
+            res.stage_ms[name] = res.stage_ms.get(name, 0.0) + e0.elapsed_time(e1)
+        return res
 
     def fetch(self, name: str, g: int) -> np.ndarray:
         """Device array of global set g as NumPy (parity tests / debugging)."""

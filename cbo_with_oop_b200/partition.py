@@ -70,3 +70,16 @@ def partition(sizes: Sequence[SetSize], world: int, tile: int = 128, snap: float
             sl.append((b, max(0, e - b)) if e > b else (0, 0))
         out.append(sl)
     return out
+
+
+def refine_owners(slices: Sequence[Sequence[Tuple[int, int]]]) -> List[int]:
+    """The rank that refines each set off the grid (SweepEngine.refine): the lowest rank whose slice of the set is
+    non-empty, or -1 when no rank holds any of it.  Every rank that touches a set holds the set's whole state, so any of
+    them could; a pure function of the partition lets every rank agree without communicating."""
+    num_sets = len(slices[0]) if slices else 0
+    owners = [-1] * num_sets
+    for r in reversed(range(len(slices))):
+        for s, (_, count) in enumerate(slices[r]):
+            if count > 0:
+                owners[s] = r
+    return owners
