@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(HERE, "..", "include")
 LIB = os.path.join(HERE, "libcbo_b200.so")
 SOURCES = ["api.cu", "tables.cu", "prior_precompute.cu", "prior_eval.cu", "prior_pair.cu", "prior_rows.cu", "posterior_fit.cu", "sweep.cu", "obs_gp_fit.cu", "sem.cu", "refine.cu", "posterior_hyper.cu"]
-HEADERS = ["cbo_common.cuh", "dmma_tile.cuh", "dmma_tma_tile.cuh", "prior_pair.cuh", "surrogate.cuh", os.path.join(INCLUDE, "cbo_b200.h")]
+HEADERS = ["cbo_common.cuh", "dmma_tile.cuh", "dmma_tma_tile.cuh", "m_triangle_pass.cuh", "prior_pair.cuh", "surrogate.cuh", os.path.join(INCLUDE, "cbo_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 

@@ -29,7 +29,7 @@
 // Roofline: FP64 pipe.  Executed flops per candidate = N^2 (+ lower order); the dense-counted figure of
 // SURVEY.md §8(d) is 2 N^2 + 2 N + d N.  Scratch traffic: each U slab is re-read once per J block
 // (~N/256 times), about 1 TB/s of L2/HBM reads chip-wide at N = 1e4 -- 15 % of HBM bandwidth.
-#include "dmma_tile.cuh"
+#include "m_triangle_pass.cuh"
 #include "prior_pair.cuh"
 
 namespace cbo {
@@ -37,7 +37,6 @@ namespace cbo {
 constexpr int kPriorWsHeader = 256;  // bytes reserved at the start of the workspace (work counter)
 
 constexpr int kPartialDoubles = 2 * CBO_PRIOR_TILE;   // one (q, m) partial per row of a work item
-constexpr int kKbPerJ = kMBlkRows / kBK;              // 16-deep k slabs per 128-column block of M
 constexpr int kPartialFloor = 1024;                    // partial slots every workspace holds, besides 4 per CTA
 
 // (this file is the grid / explicit-point evaluation, cbo_prior_eval which == 0; the interventional rows, which == 1,
@@ -49,7 +48,6 @@ __host__ __device__ inline long long prior_tiles(const cbo_set_desc& S, PriorSpl
     if (!computes_prior(S) || (sp.skip_pair && pair_eligible(S))) return 0;
     return (S.g_count + CBO_PRIOR_TILE - 1) / CBO_PRIOR_TILE;
 }
-__host__ __device__ inline int prior_nJ(const cbo_set_desc& S) { return (S.n_obs + kMBlkRows - 1) / kMBlkRows; }
 
 // Work decomposition.  chunk == 0 (the grid): one item per 128-candidate tile walks every (jb, kt) of M's lower block
 // triangle.  chunk > 0 (too few tiles to fill the GPU: small grids, small explicit-point batches): the
@@ -68,11 +66,11 @@ __host__ __device__ inline long long prior_F(int jb, int chunk) { return prior_G
 // Fallback when a launch has too few tiles to fill the GPU but too many for segments to fit the partial buffer: the
 // column blocks are dealt to `ns` items per tile, folded (jb mod 2ns in {sp, 2ns-1-sp}) so the triangular cost balances.
 __host__ __device__ inline int prior_nsplit(const cbo_set_desc& S, int nsplit) {
-    const int nJ = prior_nJ(S), cap = nJ / 2 > 1 ? nJ / 2 : 1;
+    const int nJ = m_row_blocks(S), cap = nJ / 2 > 1 ? nJ / 2 : 1;
     return nsplit < cap ? nsplit : cap;
 }
 __host__ __device__ inline long long prior_items_per_tile(const cbo_set_desc& S, PriorSplit sp) {
-    return sp.chunk > 0 ? prior_F(prior_nJ(S), sp.chunk) : prior_nsplit(S, sp.nsplit);
+    return sp.chunk > 0 ? prior_F(m_row_blocks(S), sp.chunk) : prior_nsplit(S, sp.nsplit);
 }
 __host__ __device__ inline long long prior_items(const cbo_set_desc& S, PriorSplit sp) {
     return prior_tiles(S, sp) * prior_items_per_tile(S, sp);
@@ -115,7 +113,7 @@ struct PriorItem {
     // end of the k loop: padding slabs are skipped by the producer and the consumers alike (U and M are exactly zero there,
     // so nothing changes but the stage count: 7 instead of 8 at N = 100); phase 1 still fills them for the epilogue's reads
     template <bool SPLIT> __device__ __forceinline__ int kend(int jb) const {
-        const int e = SPLIT ? kt1 : (jb + 1) * kKbPerJ;
+        const int e = SPLIT ? kt1 : (jb + 1) * kSlabsPerBlock;
         return e < kmax ? e : kmax;
     }
 };
@@ -144,7 +142,7 @@ __device__ __forceinline__ PriorItem decode_prior_item(const cbo_set_desc* __res
     }
     PriorItem it;
     it.S = sets + s;
-    it.nJ = prior_nJ(sets[s]);
+    it.nJ = m_row_blocks(sets[s]);
     it.kmax = (sets[s].n_obs + kBK - 1) / kBK;
     it.split = chunk > 0;
     it.sp = 0, it.ns = 1;
@@ -168,9 +166,9 @@ __device__ __forceinline__ PriorItem decode_prior_item(const cbo_set_desc* __res
     it.jb0 = jb, it.jb1 = jb + 1;
     if (piece < lower) {                         // strictly-lower piece: column blocks [piece*chunk, min(jb, (piece+1)*chunk))
         const int b1 = (piece + 1) * chunk < jb ? (piece + 1) * chunk : jb;
-        it.kt0 = piece * chunk * kKbPerJ, it.kt1 = b1 * kKbPerJ;
+        it.kt0 = piece * chunk * kSlabsPerBlock, it.kt1 = b1 * kSlabsPerBlock;
     } else {                                     // the diagonal block
-        it.kt0 = jb * kKbPerJ, it.kt1 = (jb + 1) * kKbPerJ;
+        it.kt0 = jb * kSlabsPerBlock, it.kt1 = (jb + 1) * kSlabsPerBlock;
     }
     return it;
 }
@@ -191,7 +189,7 @@ __device__ __forceinline__ void consume_ragged_block(const PriorItem& it, const 
                                                      int warp, int lane) {
     constexpr int BM = Cfg::BM, BN = Cfg::BN, WN = Cfg::WN, STAGES = Cfg::STAGES;
     static_assert(MW * NW * 32 == Cfg::NCONS && MW * MA2 * 8 == BM && NW <= WN, "re-tiling must cover the 128 rows with all consumer warps");
-    const int jb = it.nJ - 1, noff = jb * kKbPerJ, ke = it.kmax;   // (kmax <= nJ * 8: the padding slabs are skipped)
+    const int jb = it.nJ - 1, noff = jb * kSlabsPerBlock, ke = it.kmax;   // (kmax <= nJ * 8: the padding slabs are skipped)
     const int row0 = (warp / NW) * MA2 * 8, wn2 = warp % NW, col0 = wn2 * NB2 * 8;
     double acc[MA2][NB2][2];
 #pragma unroll
@@ -250,7 +248,7 @@ __device__ __forceinline__ void consume_item(const PriorItem& it, const double* 
                                              const double* __restrict__ scratch, const double* __restrict__ w, int warp, int lane,
                                              int ragged_cols) {
     constexpr int BM = Cfg::BM, BN = Cfg::BN, MA = Cfg::MA, NB = Cfg::NB, WN = Cfg::WN, STAGES = Cfg::STAGES;
-    static_assert(BN / kBK == kKbPerJ, "J block width");
+    static_assert(BN / kBK == kSlabsPerBlock, "J block width");
     const int wm = warp / WN, wn = warp % WN;
     const int row0 = wm * MA * 8, col0 = wn * NB * 8;
     if constexpr (LIVE == 0) {
@@ -279,7 +277,7 @@ __device__ __forceinline__ void consume_item(const PriorItem& it, const double* 
 #pragma unroll 1
     for (int jb = it.jb0; jb < jend; ++jb) {
         if (!it.mine(jb)) continue;
-        const int kb = it.template kbeg<SPLIT>(jb), ke = it.template kend<SPLIT>(jb), noff = jb * kKbPerJ;   // noff: first slab of the diagonal block
+        const int kb = it.template kbeg<SPLIT>(jb), ke = it.template kend<SPLIT>(jb), noff = jb * kSlabsPerBlock;   // noff: first slab of the diagonal block
         auto double_acc = [&]() {   // strictly-lower blocks appear twice in u^T M u
 #pragma unroll
             for (int mi = 0; mi < LV; ++mi)
@@ -417,9 +415,9 @@ prior_eval_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, PriorSpli
             const int Npad = S.n_obs_pad;
             // 16-wide column slabs of U the item touches: all of them, or (split item) its k range [kt0, kt1) followed,
             // for a segment below the diagonal, by the 8 slabs of column block jb that the epilogue dots with
-            const int nk_item = SPLIT ? it.kt1 - it.kt0 : it.nJ * kKbPerJ;
-            const bool extra = SPLIT && it.kt1 <= it.jb0 * kKbPerJ;
-            const int nKT = nk_item + (extra ? kKbPerJ : 0);
+            const int nk_item = SPLIT ? it.kt1 - it.kt0 : it.nJ * kSlabsPerBlock;
+            const bool extra = SPLIT && it.kt1 <= it.jb0 * kSlabsPerBlock;
+            const int nKT = nk_item + (extra ? kSlabsPerBlock : 0);
             // live rows of this item (the last tile of a slice and the interventional rows fill only part of the 128):
             // rows past them are never generated, multiplied or stored (rows of U are independent in U*M)
             const long long left = gcnt - (long long)it.tile * BM;
@@ -482,7 +480,7 @@ prior_eval_kernel(const cbo_set_desc* __restrict__ sets, int num_sets, PriorSpli
                 }
 #pragma unroll 1
                 for (int ks = 0; ks < nKT; ++ks) {                  // ks: slab inside the scratch
-                    const int kt = !SPLIT ? ks : (ks < nk_item ? it.kt0 + ks : it.jb0 * kKbPerJ + (ks - nk_item));
+                    const int kt = !SPLIT ? ks : (ks < nk_item ? it.kt0 + ks : it.jb0 * kSlabsPerBlock + (ks - nk_item));
                     double2 v[UW];
 #pragma unroll
                     for (int x = 0; x < UW; ++x) {
@@ -633,7 +631,7 @@ double prior_eval_flops_impl(const cbo_set_desc* h_sets, int num_sets, int num_s
                 }
             fl += 2.0 * 64.0 * blocks * g.s_count * (double)g.Kslabs * kBK;
         } else {
-            const int nJ = prior_nJ(S), lc = S.n_obs - (nJ - 1) * kMBlkRows;
+            const int nJ = m_row_blocks(S), lc = S.n_obs - (nJ - 1) * kMBlkRows;
             const int last_cols = (nJ == 1 || lc > 64) ? 128 : (lc <= 16 ? 16 : (lc <= 32 ? 32 : 64));
             const double n16 = (double)((S.n_obs + kBK - 1) / kBK * kBK);
             fl += (double)S.g_count * 2.0 * (128.0 * 128.0 * (nJ - 1) * nJ / 2.0 + last_cols * n16);
@@ -691,7 +689,7 @@ int prior_eval_impl(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int 
     if (tiles < 2 * ctas) {
         int nJmax = 1;
         for (int s = 0; s < num_sets; ++s)
-            if (prior_tiles(h_sets[s], split) > 0 && prior_nJ(h_sets[s]) > nJmax) nJmax = prior_nJ(h_sets[s]);
+            if (prior_tiles(h_sets[s], split) > 0 && m_row_blocks(h_sets[s]) > nJmax) nJmax = m_row_blocks(h_sets[s]);
         const long long budget = (long long)prior_partial_items(ctas) < 4 * ctas ? (long long)prior_partial_items(ctas) : 4 * ctas;
         for (int c = 1; c <= nJmax && nJmax > 1; ++c)
             if (count(PriorSplit{c, 1, split.skip_pair}) <= budget) { split.chunk = c; break; }

@@ -17,24 +17,18 @@
 //  * shape.  There are at most 128 rows: the work is one pass over M (HBM-bound for the single row a post-intervention
 //    trial appends: 8 N^2 / 2 bytes), not a GEMM.
 //
-// Decomposition (no atomics, deterministic): grid = (k chunk, row block I of M, set x row pass).  A CTA owns the 128 rows
-// n of block I and a run of <= 32 of the block's 16-deep k slabs of M's lower block triangle (slabs left of the diagonal
-// block count twice), streamed through a 3-stage shared-memory ring by TMA bulk copies; thread n accumulates s_n[r] = sum_k M[n][k] u_r[k] for up to 32 interventional rows r in
-// registers, then the CTA reduces sum_n u_r[n] s_n[r] and writes one (q, m) double-double partial per row;
-// prior_rows_finalize_kernel adds the partials in index order.
-#include "dmma_tile.cuh"
+// The pass over M is the shared one of m_triangle_pass.cuh, with grid z = set x row pass.  Thread n accumulates
+// s_n[r] = sum_k M[n][k] u_r[k] for up to RMAX interventional rows r in registers, then the CTA reduces sum_n u_r[n] s_n[r]
+// and writes one (q, m) double-double partial per row; prior_rows_finalize_kernel adds the partials in index order.
+#include "m_triangle_pass.cuh"
 
 namespace cbo {
 
-constexpr int kRowsSlabs = 32;     // 16-deep k slabs per CTA
-constexpr int kRowsThreads = kMBlkRows;
 constexpr int kRowsPartial = 4;    // doubles per (item, row): q_hi, q_lo, m_hi, m_lo
 // interventional rows whose accumulators live in registers at once: 32 for a whole set (register-bound, 2 CTAs per SM, the
 // arithmetic dominates), 4 for the row or two a post-intervention trial appends (6+ CTAs per SM: enough slabs in flight
 // to stream M at HBM speed)
 constexpr int kRowsWide = 32, kRowsNarrow = 4;
-constexpr int kRowsStages = 3;     // 16 KB slabs of M in flight per CTA (TMA bulk copies into a shared-memory ring)
-constexpr size_t kRowsRingBytes = (size_t)kRowsStages * kMBlkDoubles * sizeof(double);
 
 // error-free transformations; the intrinsics keep the compiler from contracting or re-associating them
 __device__ __forceinline__ void two_sum(double a, double b, double& s, double& e) {
@@ -65,7 +59,6 @@ __device__ __forceinline__ void dd_add(double h, double l, double& s, double& c)
 __host__ __device__ inline int rows_first(const cbo_set_desc& S) {
     return (S.int_row_begin > 0 && S.int_row_begin < S.n_int) ? S.int_row_begin : 0;
 }
-__host__ __device__ inline int rows_nJ(const cbo_set_desc& S) { return (S.n_obs + kMBlkRows - 1) / kMBlkRows; }
 
 struct RowsShape { int passes, nJ, chunks, rmax; };   // grid extents shared by every set of a launch (maxima); rows per pass
 __host__ __device__ inline size_t rows_partial_index(const RowsShape& sh, int set, int pass, int I, int c) {
@@ -73,79 +66,46 @@ __host__ __device__ inline size_t rows_partial_index(const RowsShape& sh, int se
 }
 
 template <int RMAX>
-__global__ void __launch_bounds__(kRowsThreads)
+__global__ void __launch_bounds__(kPassThreads)
 prior_rows_kernel(const cbo_set_desc* __restrict__ sets, RowsShape sh, double* __restrict__ partials) {
     const int set = blockIdx.z / sh.passes, pass = blockIdx.z % sh.passes;
     const cbo_set_desc& S = sets[set];
     if (!computes_prior(S)) return;
-    const int I = blockIdx.y, c = blockIdx.x;
-    const int nslab = (I + 1) * (kMBlkRows / kBK);          // k slabs of row block I inside the lower block triangle
-    const int kt0 = c * kRowsSlabs;
     const int r0 = rows_first(S) + pass * RMAX;
-    if (I >= rows_nJ(S) || kt0 >= nslab || r0 >= S.n_int) return;
-    const int kt1 = kt0 + kRowsSlabs < nslab ? kt0 + kRowsSlabs : nslab;
+    MPassItem it;
+    if (!m_pass_item(S, it) || r0 >= S.n_int) return;
     const int R = S.n_int - r0 < RMAX ? S.n_int - r0 : RMAX;
     const int Npad = S.n_obs_pad, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int diag0 = I * (kMBlkRows / kBK);                 // first slab of the diagonal block
     const double* __restrict__ U = S.u_int + (size_t)r0 * Npad;
 
-    extern __shared__ __align__(128) unsigned char ring_raw[];
-    double* sM = reinterpret_cast<double*>(ring_raw);        // [kRowsStages][128 x 16 slab, fragment order]
-    __shared__ uint64_t full[kRowsStages];
     __shared__ double su[2][RMAX][kBK];                      // u_r[k] of the current / next slab
-    __shared__ double sred[kRowsThreads / 32][RMAX][kRowsPartial];
+    __shared__ double sred[kPassThreads / 32][RMAX][kRowsPartial];
 
     double acc_s[RMAX], acc_c[RMAX];
 #pragma unroll
     for (int r = 0; r < RMAX; ++r) acc_s[r] = acc_c[r] = 0.0;
 
-    // M is streamed by TMA bulk copies (one contiguous 16 KB slab each, K1a's blocked layout) issued kRowsStages ahead by
-    // thread 0; the bytes in flight do not depend on the register budget, which is what an HBM-bound pass needs
-    const int nsl = kt1 - kt0;
-    auto issue = [&](int idx) {
-        const int st = idx % kRowsStages;
-        mbar_arrive_expect_tx(&full[st], (unsigned)(kMBlkDoubles * sizeof(double)));
-        bulk_g2s(sM + (size_t)st * kMBlkDoubles, S.M + mblk_base(I, kt0 + idx, Npad), (unsigned)(kMBlkDoubles * sizeof(double)), &full[st]);
-    };
-    if (tid == 0) {
-        for (int st = 0; st < kRowsStages; ++st) mbar_init(&full[st], 1);
-        mbar_fence_init();
-    }
-    __syncthreads();
-    if (tid == 0)
-        for (int idx = 0; idx < kRowsStages && idx < nsl; ++idx) issue(idx);
-
     // this thread's share of a slab's u columns (R x 16 doubles over 128 threads)
-    constexpr int UPT = (RMAX * kBK + kRowsThreads - 1) / kRowsThreads;
-    auto load_u = [&](int kt, double (&dst)[UPT]) {
-#pragma unroll
-        for (int x = 0; x < UPT; ++x) {
-            const int i = tid + x * kRowsThreads;
-            dst[x] = i < R * kBK ? U[(size_t)(i / kBK) * Npad + kt * kBK + (i % kBK)] : 0.0;
-        }
-    };
-    auto store_u = [&](int buf, const double (&src)[UPT]) {
-#pragma unroll
-        for (int x = 0; x < UPT; ++x) {
-            const int i = tid + x * kRowsThreads;
-            if (i < RMAX * kBK) su[buf][i / kBK][i % kBK] = src[x];
-        }
-    };
+    constexpr int UPT = (RMAX * kBK + kPassThreads - 1) / kPassThreads;
     double un[UPT];
-    load_u(kt0, un);
-    store_u(0, un);
-    __syncthreads();
-#pragma unroll 1
-    for (int idx = 0; idx < nsl; ++idx) {
-        const int kt = kt0 + idx, cur = idx & 1, st = idx % kRowsStages;
-        const bool more = idx + 1 < nsl;
-        if (more) load_u(kt + 1, un);          // next slab's u columns in flight while this slab is consumed
-        mbar_wait(&full[st], (unsigned)(idx / kRowsStages) & 1u);
-        // this thread's row of the slab, one k4-group (32 bytes; consecutive threads -> consecutive 32-byte units) at a time:
-        // the group loop is NOT unrolled, so the fully unrolled body (RMAX rows x 4 products of ~10 instructions) stays
-        // inside the instruction cache -- unrolled over all 16 columns it was 37 % "no instruction" stalls
-        const double* slab = sM + (size_t)st * kMBlkDoubles;
-        const double scale = kt < diag0 ? 2.0 : 1.0;      // strictly-lower blocks appear twice in u^T M u (exact scaling)
+    auto load_u = [&](int kt) {
+#pragma unroll
+        for (int x = 0; x < UPT; ++x) {
+            const int i = tid + x * kPassThreads;
+            un[x] = i < R * kBK ? U[(size_t)(i / kBK) * Npad + kt * kBK + (i % kBK)] : 0.0;
+        }
+    };
+    auto store_u = [&](int buf) {
+#pragma unroll
+        for (int x = 0; x < UPT; ++x) {
+            const int i = tid + x * kPassThreads;
+            if (i < RMAX * kBK) su[buf][i / kBK][i % kBK] = un[x];
+        }
+    };
+    // this thread's row of the slab, one k4-group (32 bytes; consecutive threads -> consecutive 32-byte units) at a time:
+    // the group loop is NOT unrolled, so the fully unrolled body (RMAX rows x 4 products of ~10 instructions) stays
+    // inside the instruction cache -- unrolled over all 16 columns it was 37 % "no instruction" stalls
+    auto consume = [&](const double* slab, double scale, int cur) {
 #pragma unroll 1
         for (int g = 0; g < kBK / 4; ++g) {
             const double2 a = *reinterpret_cast<const double2*>(slab + ((g * kMBlkRows + tid) << 2));
@@ -159,15 +119,13 @@ prior_rows_kernel(const cbo_set_desc* __restrict__ sets, RowsShape sh, double* _
                 }
             }
         }
-        if (more) store_u(cur ^ 1, un);   // the other buffer was last read one iteration ago, before that iteration's barrier
-        __syncthreads();                   // every thread has read ring stage st and su[cur]
-        if (tid == 0 && idx + kRowsStages < nsl) issue(idx + kRowsStages);
-    }
+    };
+    m_pass_stream(it, S.M, Npad, load_u, store_u, consume);
 
     // q partial of row r: sum over the block's rows n of u_r[n] * s_n[r]; m partial (once per row block: the CTA that
     // owns the first slab of the diagonal block): sum_n u_r[n] w[n]
-    const bool with_m = kt0 <= diag0 && diag0 < kt1;
-    const int n = I * kMBlkRows + tid;
+    const bool with_m = it.kt0 <= it.diag0 && it.diag0 < it.kt1;
+    const int n = it.I * kMBlkRows + tid;
     const double wn = with_m ? S.w[n] : 0.0;
 #pragma unroll
     for (int r = 0; r < RMAX; ++r) {
@@ -191,11 +149,11 @@ prior_rows_kernel(const cbo_set_desc* __restrict__ sets, RowsShape sh, double* _
     if (tid < RMAX) {
         double qh = 0.0, ql = 0.0, mh = 0.0, ml = 0.0;
 #pragma unroll
-        for (int wq = 0; wq < kRowsThreads / 32; ++wq) {
+        for (int wq = 0; wq < kPassThreads / 32; ++wq) {
             dd_add(sred[wq][tid][0], sred[wq][tid][1], qh, ql);
             dd_add(sred[wq][tid][2], sred[wq][tid][3], mh, ml);
         }
-        double* out = partials + rows_partial_index(sh, set, pass, I, c) + tid * kRowsPartial;
+        double* out = partials + rows_partial_index(sh, set, pass, it.I, it.c) + tid * kRowsPartial;
         out[0] = qh, out[1] = ql, out[2] = mh, out[3] = ml;
     }
 }
@@ -214,11 +172,11 @@ prior_rows_finalize_kernel(const cbo_set_desc* __restrict__ sets, RowsShape sh, 
     if (!computes_prior(S)) return;      // CTA-uniform
     const int r = rows_first(S) + pass * sh.rmax + row;
     double qh = 0.0, ql = 0.0, mh = 0.0, ml = 0.0;
-    const int nJ = rows_nJ(S);
+    const int nJ = m_row_blocks(S);
     if (r < S.n_int) {                   // warp-uniform
         for (int e = sub * 32 + lane; e < nJ * sh.chunks; e += 32 * wpr) {
             const int I = e / sh.chunks, c = e - I * sh.chunks;
-            if (c * kRowsSlabs >= (I + 1) * (kMBlkRows / kBK)) continue;     // the item does not exist (nothing was written)
+            if (!m_item_exists(I, c)) continue;
             const double* p = partials + rows_partial_index(sh, set, pass, I, c) + row * kRowsPartial;
             dd_add(p[0], p[1], qh, ql);
             dd_add(p[2], p[3], mh, ml);
@@ -244,16 +202,12 @@ prior_rows_finalize_kernel(const cbo_set_desc* __restrict__ sets, RowsShape sh, 
 }
 
 static RowsShape rows_shape(const cbo_set_desc* h_sets, int num_sets) {
-    RowsShape sh{0, 0, 0, kRowsWide};
+    const dim3 g = m_pass_grid(h_sets, num_sets, 1);
+    RowsShape sh{0, (int)g.y, (int)g.x, kRowsWide};
     int rows_max = 0;
     for (int s = 0; s < num_sets; ++s) {
-        const cbo_set_desc& S = h_sets[s];
-        if (!computes_prior(S)) continue;
-        const int rows = S.n_int - rows_first(S), nJ = rows_nJ(S);
-        const int chunks = (nJ * (kMBlkRows / kBK) + kRowsSlabs - 1) / kRowsSlabs;
-        if (rows > rows_max) rows_max = rows;
-        if (nJ > sh.nJ) sh.nJ = nJ;
-        if (chunks > sh.chunks) sh.chunks = chunks;
+        const int rows = h_sets[s].n_int - rows_first(h_sets[s]);
+        if (computes_prior(h_sets[s]) && rows > rows_max) rows_max = rows;
     }
     if (rows_max == 0) return sh;
     sh.rmax = rows_max <= kRowsNarrow ? kRowsNarrow : kRowsWide;
@@ -278,13 +232,11 @@ int prior_rows_impl(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int 
     CBO_REQUIRE(d_ws != nullptr && ws_bytes >= ws_offset + need,
                 "cbo_prior_eval: workspace of %zu bytes is too small for the interventional rows (%zu needed); see "
                 "cbo_prior_workspace_bytes", ws_bytes, ws_offset + need);
-    CBO_REQUIRE((long long)num_sets * sh.passes <= 65535, "cbo_prior_eval: too many sets for one launch");
     double* partials = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(d_ws) + ws_offset);
     const dim3 grid(sh.chunks, sh.nJ, num_sets * sh.passes);
-    CBO_CUDA(allow_dynamic_smem(prior_rows_kernel<kRowsNarrow>, kRowsRingBytes));
-    CBO_CUDA(allow_dynamic_smem(prior_rows_kernel<kRowsWide>, kRowsRingBytes));
-    if (sh.rmax == kRowsNarrow) prior_rows_kernel<kRowsNarrow><<<grid, kRowsThreads, kRowsRingBytes, st>>>(d_sets, sh, partials);
-    else prior_rows_kernel<kRowsWide><<<grid, kRowsThreads, kRowsRingBytes, st>>>(d_sets, sh, partials);
+    const auto kernel = sh.rmax == kRowsNarrow ? prior_rows_kernel<kRowsNarrow> : prior_rows_kernel<kRowsWide>;
+    if (int rc = m_pass_prepare(kernel, grid, "cbo_prior_eval")) return rc;
+    kernel<<<grid, kPassThreads, kPassRingBytes, st>>>(d_sets, sh, partials);
     note_launch();
     CBO_CUDA(cudaGetLastError());
     prior_rows_finalize_kernel<<<num_sets * sh.passes, dim3(32, kRowsWide), 0, st>>>(d_sets, sh, partials);

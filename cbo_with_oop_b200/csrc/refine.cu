@@ -15,9 +15,8 @@
 //   acquisition     u = (best - mu) / sd,  ei = sign sd (u Phi + phi),  dei = -sign Phi dmu + sign phi dvar / (2 sd)
 //                   c = cost_fix + cost_variable sum |x_k|,  acq = ei / c,  dacq = (dei - acq dc) / c
 //
-// Prior-gradient pass (refine_prior_kernel): the model is K1c (prior_rows.cu).  A CTA owns the 128 rows n of a row block
-// of M and a run of <= kRefSlabs of the block's 16-deep column slabs of M's lower block triangle, streamed by TMA bulk
-// copies through a 3-stage ring.  For each of the 8 points of a set, thread n accumulates
+// Prior-gradient pass (refine_prior_kernel): the shared pass over M of m_triangle_pass.cuh, with grid z = set x batch of
+// 8 points.  For each of the 8 points of a set, thread n accumulates
 //   S_u[n] = sum_k sc M_nk u_k  and  S_a,i[n] = sum_k sc M_nk a_ik      (sc = 2 left of the diagonal block, 1 inside it)
 // and the CTA reduces  q = sum_n u_n S_u[n],  dv_i = sum_n (a_in S_u[n] + u_n S_a,i[n])  (the symmetric form of 2 a_i^T M u
 // over the lower block triangle) and, once per row block, u.w and a_i.w.  That is 1 + d FMAs per element of M and point;
@@ -31,18 +30,14 @@
 // the 8 trial points of the next pass are clamp(x + 2^-j p), j = 0..7, accepted by Armijo's rule.  The first direction is
 // the gradient scaled so that its largest move is one grid spacing.
 #include <float.h>
-#include "dmma_tile.cuh"
+#include "m_triangle_pass.cuh"
 #include "surrogate.cuh"
 
 namespace cbo {
 
 constexpr int kRefB = 8;                       // trial points per set and pass
-constexpr int kRefSlabs = 32;                  // 16-deep slabs of M per CTA of the prior pass
-constexpr int kRefStages = 3;                  // 16 KB slabs in flight per CTA
-constexpr int kRefThreads = kMBlkRows;         // prior pass: thread n owns row n of a row block
 constexpr int kRefPF = 2 + 2 * CBO_MAX_D;      // partial per (item, point): m, q, a.w [4], dv [4]
 constexpr int kStepThreads = 32 * kRefB;       // step / gradient kernels: one warp per point
-constexpr size_t kRefRingBytes = (size_t)kRefStages * kMBlkDoubles * sizeof(double);
 constexpr double kArmijo = 1e-4;
 
 struct RefineState {                           // one per set, in the workspace
@@ -56,11 +51,9 @@ struct RefineState {                           // one per set, in the workspace
     int32_t running, iter, status, ntrial, qn, max_iter;
 };
 
-__host__ __device__ inline int ref_nJ(const cbo_set_desc& S) { return (S.n_obs + kMBlkRows - 1) / kMBlkRows; }
-__host__ __device__ inline int ref_chunks(const cbo_set_desc& S) { return (ref_nJ(S) * (kMBlkRows / kBK) + kRefSlabs - 1) / kRefSlabs; }
 // partial slots of one batch of 8 points of a set
 __host__ __device__ inline long long ref_items(const cbo_set_desc& S) {
-    return computes_prior(S) ? (long long)ref_nJ(S) * ref_chunks(S) : 0;
+    return computes_prior(S) ? (long long)m_row_blocks(S) * m_chunks(S) : 0;
 }
 constexpr long long kRefItemDoubles = (long long)kRefB * kRefPF;
 constexpr size_t kRefHeader = 256;             // [0]: sets still running (int32)
@@ -76,26 +69,19 @@ struct PassArgs {
 };
 
 template <int D>
-__global__ void __launch_bounds__(kRefThreads)
+__global__ void __launch_bounds__(kPassThreads)
 refine_prior_kernel(const cbo_set_desc* __restrict__ sets, PassArgs a) {
     const int set = blockIdx.z / a.nbatch, batch = blockIdx.z % a.nbatch;
     const cbo_set_desc& S = sets[set];
     if (S.d != D || !computes_prior(S)) return;
     if (a.state && !a.state[set].running) return;
-    const int nJ = ref_nJ(S), chunks = ref_chunks(S);
-    const int I = blockIdx.y, c = blockIdx.x;
-    const int nslab = (I + 1) * (kMBlkRows / kBK), kt0 = c * kRefSlabs;
-    if (I >= nJ || c >= chunks || kt0 >= nslab) return;
-    const int kt1 = kt0 + kRefSlabs < nslab ? kt0 + kRefSlabs : nslab;
-    const int nsl = kt1 - kt0, diag0 = I * (kMBlkRows / kBK);
+    MPassItem it;
+    if (!m_pass_item(S, it)) return;
     const int N = S.n_obs, Npad = S.n_obs_pad, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
-    extern __shared__ __align__(128) unsigned char ring_raw[];
-    double* sM = reinterpret_cast<double*>(ring_raw);
-    __shared__ uint64_t full[kRefStages];
     __shared__ __align__(16) double tab[2][kRefB][1 + D][kBK];      // u (row 0) and a_k (rows 1..D) of the slab's columns
     __shared__ double sx[kRefB][D];
-    __shared__ double sred[kRefThreads / 32][kRefB][2 + 2 * D];
+    __shared__ double sred[kPassThreads / 32][kRefB][2 + 2 * D];
     double il[D];
 #pragma unroll
     for (int k = 0; k < D; ++k) il[k] = 1.0 / S.ls_int[k];
@@ -105,23 +91,12 @@ refine_prior_kernel(const cbo_set_desc* __restrict__ sets, PassArgs a) {
         int pi = batch * kRefB + q;
         if (pi >= a.npts) pi = a.npts - 1;          // padding points repeat the last one (their partials are not read)
         sx[q][k] = a.pts[a.set_stride * set + (long long)pi * a.pt_stride + k];
-    }
-    if (tid == 0) {
-        for (int st = 0; st < kRefStages; ++st) mbar_init(&full[st], 1);
-        mbar_fence_init();
-    }
-    __syncthreads();
-    auto issue = [&](int idx) {
-        const int st = idx % kRefStages;
-        mbar_arrive_expect_tx(&full[st], (unsigned)(kMBlkDoubles * sizeof(double)));
-        bulk_g2s(sM + (size_t)st * kMBlkDoubles, S.M + mblk_base(I, kt0 + idx, Npad), (unsigned)(kMBlkDoubles * sizeof(double)), &full[st]);
-    };
-    if (tid == 0)
-        for (int idx = 0; idx < kRefStages && idx < nsl; ++idx) issue(idx);
+    }   // (sx is published by the barrier that follows the ring's set-up)
 
     // table entry of this thread: point tid / 16, column tid % 16 of slab kt
     const int tq = tid >> 4, tc = tid & 15;
-    auto entry = [&](int kt, double (&e)[1 + D]) {
+    double en[1 + D];
+    auto entry = [&](int kt) {
         const int col = kt * kBK + tc;
         if (col < N) {
             double r2 = 0.0, z[D];
@@ -130,35 +105,24 @@ refine_prior_kernel(const cbo_set_desc* __restrict__ sets, PassArgs a) {
                 z[k] = (sx[tq][k] - S.x_obs_int[(size_t)k * N + col]) * il[k];
                 r2 = fma(z[k], z[k], r2);
             }
-            e[0] = exp(-0.5 * r2);
+            en[0] = exp(-0.5 * r2);
 #pragma unroll
-            for (int k = 0; k < D; ++k) e[1 + k] = e[0] * z[k] * il[k];
+            for (int k = 0; k < D; ++k) en[1 + k] = en[0] * z[k] * il[k];
         } else {
 #pragma unroll
-            for (int k = 0; k <= D; ++k) e[k] = 0.0;
+            for (int k = 0; k <= D; ++k) en[k] = 0.0;
         }
     };
-    auto store = [&](int buf, const double (&e)[1 + D]) {
+    auto store = [&](int buf) {
 #pragma unroll
-        for (int k = 0; k <= D; ++k) tab[buf][tq][k][tc] = e[k];
+        for (int k = 0; k <= D; ++k) tab[buf][tq][k][tc] = en[k];
     };
     double acc[kRefB][1 + D];
 #pragma unroll
     for (int q = 0; q < kRefB; ++q)
 #pragma unroll
         for (int k = 0; k <= D; ++k) acc[q][k] = 0.0;
-    double en[1 + D];
-    entry(kt0, en);
-    store(0, en);
-    __syncthreads();
-#pragma unroll 1
-    for (int idx = 0; idx < nsl; ++idx) {
-        const int kt = kt0 + idx, cur = idx & 1, st = idx % kRefStages;
-        const bool more = idx + 1 < nsl;
-        if (more) entry(kt + 1, en);
-        mbar_wait(&full[st], (unsigned)(idx / kRefStages) & 1u);
-        const double* slab = sM + (size_t)st * kMBlkDoubles;
-        const double scale = kt < diag0 ? 2.0 : 1.0;
+    auto consume = [&](const double* slab, double scale, int cur) {
 #pragma unroll 1
         for (int g = 0; g < kBK / 4; ++g) {
             const double2 m01 = *reinterpret_cast<const double2*>(slab + ((g * kMBlkRows + tid) << 2));
@@ -179,14 +143,12 @@ refine_prior_kernel(const cbo_set_desc* __restrict__ sets, PassArgs a) {
                 }
             }
         }
-        if (more) store(cur ^ 1, en);
-        __syncthreads();
-        if (tid == 0 && idx + kRefStages < nsl) issue(idx + kRefStages);
-    }
+    };
+    m_pass_stream(it, S.M, Npad, entry, store, consume);
 
     // row n's share: q = u_n S_u, dv_i = a_in S_u + u_n S_a,i; once per row block (c == 0): m = u_n w_n, a_in w_n
-    const int n = I * kMBlkRows + tid;
-    const bool with_m = c == 0;
+    const int n = it.I * kMBlkRows + tid;
+    const bool with_m = it.c == 0;
     const double wn = (with_m && n < N) ? S.w[n] : 0.0;
 #pragma unroll
     for (int q = 0; q < kRefB; ++q) {
@@ -221,8 +183,8 @@ refine_prior_kernel(const cbo_set_desc* __restrict__ sets, PassArgs a) {
     }
     __syncthreads();
     double* out = a.partials + (a.state ? a.state[set].part_base : 0) +
-                  (((long long)batch * nJ + I) * chunks + c) * kRefItemDoubles;
-    for (int e = tid; e < kRefB * kRefPF; e += kRefThreads) {
+                  (((long long)batch * m_row_blocks(S) + it.I) * m_chunks(S) + it.c) * kRefItemDoubles;
+    for (int e = tid; e < kRefB * kRefPF; e += kPassThreads) {
         const int q = e / kRefPF, f = e % kRefPF;
         // slot layout per point: m, q, a.w[CBO_MAX_D], dv[CBO_MAX_D]
         double s = 0.0;
@@ -273,13 +235,13 @@ __device__ void eval_point(const cbo_set_desc& S, const RefSmem& sm, const doubl
     double m = 0.0, v = 0.0, dm[CBO_MAX_D] = {0.0, 0.0, 0.0, 0.0}, dv[CBO_MAX_D] = {0.0, 0.0, 0.0, 0.0};
     if (partials) {
         // partial slots in index order per lane, then a fixed butterfly: the same additions on every run
-        const int chunks = ref_chunks(S), items = ref_nJ(S) * chunks;
+        const int chunks = m_chunks(S), items = m_row_blocks(S) * chunks;
         double acc[kRefPF];
 #pragma unroll
         for (int f = 0; f < kRefPF; ++f) acc[f] = 0.0;
         for (int e = lane; e < items; e += 32) {
             const int I = e / chunks, c = e - I * chunks;
-            if (c * kRefSlabs >= (I + 1) * (kMBlkRows / kBK)) continue;
+            if (!m_item_exists(I, c)) continue;
             const double* p = partials + (long long)e * kRefItemDoubles + q * kRefPF;
 #pragma unroll
             for (int f = 0; f < kRefPF; ++f) acc[f] += p[f];
@@ -595,27 +557,17 @@ size_t refine_workspace_bytes_impl(const cbo_set_desc* h_sets, int num_sets) {
 
 // one prior-gradient pass: a launch per dimension count present among the sets with a device prior
 static int launch_prior_pass(const cbo_set_desc* h_sets, const cbo_set_desc* d_sets, int num_sets, const PassArgs& a, cudaStream_t st) {
-    int nJ = 0, chunks = 0;
-    bool dims[CBO_MAX_D + 1] = {};
-    for (int s = 0; s < num_sets; ++s) {
-        const cbo_set_desc& S = h_sets[s];
-        if (!computes_prior(S)) continue;
-        dims[S.d] = true;
-        if (ref_nJ(S) > nJ) nJ = ref_nJ(S);
-        if (ref_chunks(S) > chunks) chunks = ref_chunks(S);
+    const dim3 grid = m_pass_grid(h_sets, num_sets, a.nbatch);
+    void (*const kernels[])(const cbo_set_desc*, PassArgs) = {refine_prior_kernel<1>, refine_prior_kernel<2>, refine_prior_kernel<3>, refine_prior_kernel<4>};
+    for (int d = 1; d <= CBO_MAX_D; ++d) {
+        bool present = false;
+        for (int s = 0; s < num_sets; ++s) present |= computes_prior(h_sets[s]) && h_sets[s].d == d;
+        if (!present) continue;
+        if (int rc = m_pass_prepare(kernels[d - 1], grid, "K7")) return rc;
+        kernels[d - 1]<<<grid, kPassThreads, kPassRingBytes, st>>>(d_sets, a);
+        note_launch();
+        CBO_CUDA(cudaGetLastError());
     }
-    if (!nJ) return 0;
-    CBO_REQUIRE((long long)num_sets * a.nbatch <= 65535 && nJ <= 65535, "K7: too many sets or rows for one launch");
-    const dim3 grid(chunks, nJ, num_sets * a.nbatch);
-#define CBO_REF_PASS(D)                                                                                   \
-    if (dims[D]) {                                                                                        \
-        CBO_CUDA(allow_dynamic_smem(refine_prior_kernel<D>, kRefRingBytes));                              \
-        refine_prior_kernel<D><<<grid, kRefThreads, kRefRingBytes, st>>>(d_sets, a);                      \
-        note_launch();                                                                                    \
-        CBO_CUDA(cudaGetLastError());                                                                     \
-    }
-    CBO_REF_PASS(1) CBO_REF_PASS(2) CBO_REF_PASS(3) CBO_REF_PASS(4)
-#undef CBO_REF_PASS
     return 0;
 }
 
