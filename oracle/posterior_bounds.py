@@ -256,7 +256,7 @@ def posterior_ref_block(X, m, v, st, path, separable=False):
     base = LD(st["s2"]) + v.astype(LD)
     var = (base - ss) + LD(VAR_NOISE)
     e_var = e_ss + SLACK * U * (np.abs(a) + np.abs(base - ss).astype(np.float64) + np.abs(var).astype(np.float64))
-    return dict(mu=mu, var=var, e_mu=e_mu, e_var=e_var, ss=ss.astype(np.float64), n=n)
+    return dict(mu=mu, var=var, e_mu=e_mu, e_var=e_var, ss=ss.astype(np.float64), n=n, t=t, dt=dt)
 
 
 def check_posterior(mu, var, ref):
@@ -269,8 +269,9 @@ def check_posterior(mu, var, ref):
 # --------------------------------------------------------------------------------------------------
 # EI, acq
 # --------------------------------------------------------------------------------------------------
-def ei_bound(best, mu, var, task_sign):
-    """Bound on |EI^ - EI(best, mu, var)| of the kernel's expected_improvement at its own (mu, var) (module docstring)."""
+def ei_terms(best, mu, var):
+    """sd, u, phi(u), Phi(u) at the kernel's own (mu, var) and the first-order relative errors eps_u, eps_phi, eps_Phi of
+    the kernel's u, phi and Phi (module docstring), as float64 arrays."""
     from scipy.special import erfc, erfcx, ndtr
     mu, var = np.asarray(mu, np.float64), np.asarray(var, np.float64)
     with np.errstate(all="ignore"):
@@ -285,6 +286,14 @@ def ei_bound(best, mu, var, task_sign):
         eps_u = 3.0 * U
         eps_phi = 0.5 * u * u * (2.0 * eps_u + U) + (2 * EXP_ULP + 2) * U
         eps_Phi = kappa * (eps_u + 2.0 * U) + 2 * ERFC_ULP * U
+    return dict(sd=sd, u=u, phi=phi, Phi=Phi, eps_u=eps_u, eps_phi=eps_phi, eps_Phi=eps_Phi)
+
+
+def ei_bound(best, mu, var, task_sign):
+    """Bound on |EI^ - EI(best, mu, var)| of the kernel's expected_improvement at its own (mu, var) (module docstring)."""
+    t = ei_terms(best, mu, var)
+    sd, u, phi, Phi, eps_u, eps_phi, eps_Phi = (t[k] for k in ("sd", "u", "phi", "Phi", "eps_u", "eps_phi", "eps_Phi"))
+    with np.errstate(all="ignore"):
         g = u * Phi + phi
         dg = np.abs(u * Phi) * (eps_u + eps_Phi + U) + phi * eps_phi + U * np.abs(g)
         # (+ an absolute floor for results in or below the subnormal range: phi, Phi and EI underflow far in the tail)
